@@ -25,7 +25,7 @@ The other configurations hang off keys the driver keeps:
   config.parity_checked       in-bench parity of the timed kernels against the
                               reference's outputs (the run FAILS on mismatch)
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N
     python bench.py --impl reference      # the reference's CPU code, host cores
 """
@@ -50,6 +50,8 @@ C4_TOTAL_COLS = 4_000_000
 C1_DIM, C1_DENSITY = (20000, 5000), 0.05
 C5_NROW, C5_NCOL, C5_DENSITY = 100_000, 2_000_000, 0.01
 MIN_WARMUP = 32
+# --dump-outputs stays below 64 MB in all, .npy headers included
+DUMP_BYTES = 63 * 10**6
 METRIC = "nnz/s for SVT colSums+colMeans+rowSums+rowVars (na.rm=TRUE), " \
          "33538x1e6 int counts d=0.07 per GPU"
 OPS = ["colSums", "colMeans", "rowSums", "rowVars"]
@@ -459,6 +461,38 @@ def run_reference(args):
 
 
 # ---------------------------------------------------------------------------
+# outputs of the timed step, for comparing two builds on the same inputs
+
+def dump_outputs(path, last, rank, world):
+    """Write the results of the last timed step as <path>/<op>.npy (float64).
+    Row results are allreduced, so rank 0 writes them; every rank writes its
+    own columns (<op>_rank<r>.npy when there are several).  Beyond
+    DUMP_BYTES in all, the column results are cut to the same fixed, seeded
+    sample of columns on every run."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    out = {op: np.asarray(t.cpu().numpy(), dtype=np.float64)
+           for op, t in last.items()}
+    col_ops = [op for op in OPS if op.startswith("col")]
+    row_bytes = sum(out[op].nbytes for op in OPS if op.startswith("row"))
+    ncol = out[col_ops[0]].size
+    keep = (DUMP_BYTES - row_bytes) // (8 * len(col_ops) * world)
+    pick = None
+    if ncol > keep:
+        pick = np.sort(np.random.Generator(np.random.PCG64(0)).choice(
+            ncol, size=keep, replace=False))
+    for op in OPS:
+        if op in col_ops:
+            a = out[op] if pick is None else out[op][pick]
+            name = op if world == 1 else "%s_rank%d" % (op, rank)
+        elif rank == 0:
+            a, name = out[op], op
+        else:
+            continue
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
+# ---------------------------------------------------------------------------
 # in-bench parity
 
 class ParityError(RuntimeError):
@@ -526,7 +560,13 @@ def main():
     ap.add_argument("--no-products", action="store_true")
     ap.add_argument("--no-configs", action="store_true",
                     help="skip the C1 / C5 / C4 legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step "
+                         "(colSums, colMeans, rowSums, rowVars) as "
+                         "DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -636,6 +676,13 @@ def main():
     for _ in range(warmup):
         for op in OPS:
             run_op(op)
+    # --dump-outputs: the last step's results are copied aside in stream
+    # order as they come (colSums and colMeans share col_out)
+    last = None
+    if args.dump_outputs:
+        last = {op: torch.empty(ncol if op.startswith("col") else NROW,
+                                dtype=torch.float64, device=dev)
+                for op in OPS}
     barrier()
     launches0 = N.launch_count()
     t_begin = torch.cuda.Event(enable_timing=True)
@@ -645,13 +692,18 @@ def main():
     for s in range(args.steps):
         ev[s][0].record()
         for i, op in enumerate(OPS):
-            run_op(op)
+            if last is not None and s == args.steps - 1:
+                last[op].copy_(run_op(op))
+            else:
+                run_op(op)
             ev[s][i + 1].record()
     t_end.record()
     barrier()
     wall1 = time.time()
     launches = N.launch_count() - launches0
     clocks = sampler.stop(wall0, wall1) if sampler else None
+    if last is not None:
+        dump_outputs(args.dump_outputs, last, rank, world)
     per_op_ms = [sum(ev[s][i].elapsed_time(ev[s][i + 1])
                      for s in range(args.steps)) / args.steps
                  for i in range(len(OPS))]

@@ -374,3 +374,43 @@ def matmul_cases():
                                     "double"),
                                   np.arange(1.0, 13.0).reshape(6, 2))
     return out
+
+
+# CSC <-> SVT bridges: (dtype, one_based, shuffle, zeros) of the stored cases
+# (tests/golden/csc_bridges.npz, written by tests/golden/make_csc_golden.py)
+CSC_DIM = (211, 57)
+CSC_CASES = [(np.float64, False, False, True), (np.int32, True, True, True),
+             (np.float64, True, True, False), (np.int32, False, False, False)]
+
+
+def csc_key(dtype, one_based, shuffle, zeros):
+    return "%s|%d|%d|%d" % (np.dtype(dtype).name, one_based, shuffle, zeros)
+
+
+def csc_fixture(seed, nrow, ncol, dtype, one_based, shuffle, zeros):
+    """CSC arrays with explicit zeros in @x and (optionally) unsorted row
+    indices inside the columns"""
+    rng = np.random.Generator(np.random.PCG64(seed))
+    cnt = rng.binomial(nrow, 0.2, size=ncol)
+    cnt[rng.integers(0, ncol, 3)] = 0
+    p = np.zeros(ncol + 1, dtype=np.int64)
+    np.cumsum(cnt, out=p[1:])
+    i = np.concatenate([np.sort(rng.choice(nrow, size=c, replace=False))
+                        for c in cnt] + [np.zeros(0, np.int64)]).astype(np.int32)
+    if dtype == np.float64:
+        x = np.round(rng.standard_normal(i.size), 2)
+        x[rng.random(i.size) < 0.01] = fx.NA_R
+        x[rng.random(i.size) < 0.01] = np.nan
+    else:
+        x = rng.integers(-5, 6, size=i.size).astype(np.int32)
+        x[rng.random(i.size) < 0.01] = fx.NA_I
+    if zeros:
+        x[rng.random(i.size) < 0.1] = 0
+    else:
+        x[x == 0] = 1
+    if shuffle:
+        for j in range(ncol):
+            q = rng.permutation(cnt[j])
+            i[p[j]:p[j + 1]] = i[p[j]:p[j + 1]][q]
+            x[p[j]:p[j + 1]] = x[p[j]:p[j + 1]][q]
+    return p, i + (1 if one_based else 0), x

@@ -1205,50 +1205,24 @@ def test_summarize_int_var_two_pass_form(name, monkeypatch):
 
 # ---- CSC <-> device-resident SVT bridges ------------------------------------
 
-def _csc_fixture(seed, nrow, ncol, dtype, one_based, shuffle, zeros):
-    """CSC arrays with explicit zeros in @x and (optionally) unsorted row
-    indices inside the columns"""
-    rng = np.random.Generator(np.random.PCG64(seed))
-    cnt = rng.binomial(nrow, 0.2, size=ncol)
-    cnt[rng.integers(0, ncol, 3)] = 0
-    p = np.zeros(ncol + 1, dtype=np.int64)
-    np.cumsum(cnt, out=p[1:])
-    i = np.concatenate([np.sort(rng.choice(nrow, size=c, replace=False))
-                        for c in cnt] + [np.zeros(0, np.int64)]).astype(np.int32)
-    if dtype == np.float64:
-        x = np.round(rng.standard_normal(i.size), 2)
-        x[rng.random(i.size) < 0.01] = fx.NA_R
-        x[rng.random(i.size) < 0.01] = np.nan
-    else:
-        x = rng.integers(-5, 6, size=i.size).astype(np.int32)
-        x[rng.random(i.size) < 0.01] = fx.NA_I
-    if zeros:
-        x[rng.random(i.size) < 0.1] = 0
-    else:
-        x[x == 0] = 1
-    if shuffle:
-        for j in range(ncol):
-            q = rng.permutation(cnt[j])
-            i[p[j]:p[j + 1]] = i[p[j]:p[j + 1]][q]
-            x[p[j]:p[j + 1]] = x[p[j]:p[j + 1]][q]
-    return p, i + (1 if one_based else 0), x
+CSC_GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)),
+                          "golden", "csc_bridges.npz")
 
 
-@pytest.mark.parametrize("dtype,one_based,shuffle,zeros", [
-    (np.float64, False, False, True), (np.int32, True, True, True),
-    (np.float64, True, True, False), (np.int32, False, False, False)])
+@pytest.mark.parametrize("dtype,one_based,shuffle,zeros", cases.CSC_CASES)
 def test_csc_bridges_vs_reference(dtype, one_based, shuffle, zeros):
     """C_svtgpu_from_CSC against the reference's C_build_SVT_from_CSC (zeros
     dropped, entries ordered by row, 0- / 1-based indices, integer / double
     indptr), C_svtgpu_to_CSC against its
     C_from_SVT_SparseMatrix_to_CsparseMatrix, and the statistics of the
-    handle against the reference's on the SVT it builds."""
-    from oracle import refcall
-    nrow, ncol = 211, 57
-    p, i, x = _csc_fixture(17, nrow, ncol, dtype, one_based, shuffle, zeros)
-    ref_svt = refcall.build_SVT_from_CSC((nrow, ncol), p.astype(np.int32), x,
-                                         i, one_based)
-    ep, ei, ex = refcall.from_SVT_to_CSC(ref_svt)
+    handle against the reference's on the SVT it builds (inputs and expected
+    outputs stored by tests/golden/make_csc_golden.py)."""
+    nrow, ncol = cases.CSC_DIM
+    key = cases.csc_key(dtype, one_based, shuffle, zeros) + "|"
+    with np.load(CSC_GOLDEN, allow_pickle=False) as f:
+        G = {k[len(key):]: f[k] for k in f.files if k.startswith(key)}
+    p, i, x = G["p"], G["i"], G["x"]
+    ep, ei, ex = G["ep"], G["ei"], G["ex"]
     for ip in (p.astype(np.int32), p.astype(np.float64)):
         h = sa.from_csc((nrow, ncol), ip, x, i, one_based)
         gp, gi, gx = sa.to_csc(h)
@@ -1258,7 +1232,7 @@ def test_csc_bridges_vs_reference(dtype, one_based, shuffle, zeros):
         assert sa.to_csc(h, as_ngCMatrix=True)[2] is None
         for op in ("sum", "max"):
             for na_rm in (False, True):
-                e = refcall.colStats(ref_svt, op, na_rm=na_rm).value
+                e = G["col|%s|%d" % (op, na_rm)]
                 v = np.asarray(sa.svt._colStats(op, h, na_rm=na_rm,
                                                 useNames=False))
                 if dtype == np.int32 or op == "max":
@@ -1269,7 +1243,7 @@ def test_csc_bridges_vs_reference(dtype, one_based, shuffle, zeros):
                                      np.append(np.abs(np.nan_to_num(ex)), 0),
                                      np.minimum(ep[:-1], ex.size)) *
                                  (np.diff(ep) > 0))
-                e = refcall.rowStats(ref_svt, op, na_rm=na_rm).value
+                e = G["row|%s|%d" % (op, na_rm)]
                 v = np.asarray(sa.svt._rowStats(op, h, na_rm=na_rm,
                                                 useNames=False))
                 if dtype == np.int32 or op == "max":
@@ -1280,7 +1254,6 @@ def test_csc_bridges_vs_reference(dtype, one_based, shuffle, zeros):
                                      ei, weights=np.abs(np.nan_to_num(ex)),
                                      minlength=nrow))
         h.release()
-    ref_svt.release()
     # a host SVT goes the same way: to_device() then to_CSC
     xs = sa.SVT_SparseArray((nrow, ncol), "double" if dtype == np.float64
                             else "integer", ep, ei, ex)

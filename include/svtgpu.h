@@ -327,6 +327,40 @@ int svtgpu_matmul(svtgpu_matrix *m, const void *d, int d_type, int64_t K,
 int svtgpu_matmul_dev(svtgpu_matrix *m, const void *d_d_rowmajor, int d_type,
 		      int64_t K, double *d_ans_rowmajor, void *stream);
 
+/* ---- element-wise operations that keep the implicit zeros at zero ----
+ * Arith `x * v`, `v * x`, `x / v` and the Math functions below, with base R's
+ * dense semantics (result types, NA / NaN, integer overflow: the rules live
+ * in csrc/svt_semantics.h).  *out is a NEW matrix (owned by the caller, free
+ * it with svtgpu_matrix_free()) with x's geometry; computed values equal to 0
+ * (-0 included) are dropped, NA and NaN kept; svtgpu_matrix_info(*out)
+ * reports the result type.  The result starts with no cached knowledge
+ * (value bounds, split tables, transpose).  x is not modified.
+ *   operand: host memory, operand_type SVTGPU_LGL / INT / DOUBLE, ignored for
+ *            Math ops (may be NULL);
+ *   margin:  0 = scalar (operand_len 1), 1 = operand[row] (operand_len =
+ *            nrow), 2 = operand[leaf] (operand_len = nleaf: a column shard
+ *            passes its own slice of the per-column vector);
+ *   operand_on_left: `v * x` / `v / x` (the latter is refused).
+ * An operation that would turn the implicit zeros into something else
+ * (`x * Inf`, `x * NA`, `x / 0`, `v / x`, other opcodes) fails with
+ * SVTGPU_ERR_ARG and R's wording before any device work.
+ * *warn: SVTGPU_EW_WARN_* bits. */
+#define SVTGPU_EW_MUL       1
+#define SVTGPU_EW_DIV       2
+#define SVTGPU_EW_ABS      11
+#define SVTGPU_EW_SIGN     12
+#define SVTGPU_EW_SQRT     13
+#define SVTGPU_EW_FLOOR    14
+#define SVTGPU_EW_CEILING  15
+#define SVTGPU_EW_TRUNC    16
+#define SVTGPU_EW_LOG1P    17
+#define SVTGPU_EW_EXPM1    18
+#define SVTGPU_EW_WARN_INT_OVERFLOW  1  /* "NAs produced by integer overflow" */
+#define SVTGPU_EW_WARN_NAN           2  /* "NaNs produced" */
+int svtgpu_ewise(svtgpu_matrix *x, int op, const void *operand,
+		 int operand_type, int64_t operand_len, int margin,
+		 int operand_on_left, svtgpu_matrix **out, int *warn);
+
 /* ---- synthetic data (benchmark inputs, generated in HBM) ----
  * Counter-based, so any leaf can be regenerated anywhere: with
  *   h  = mix64(seed + (cell + 1) * 0x9E3779B97F4A7C15),  cell = leaf*nrow + i

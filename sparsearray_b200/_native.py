@@ -100,7 +100,16 @@ SIGNATURES = {
     "svtgpu_gen_fill": (_INT, [_I64, _I64, _I64, _c.c_uint64, _c.c_uint32,
                                _c.c_uint32, _P, _INT, _INT, _P, _P, _P, _P]),
     "svtgpu_exclusive_scan": (_INT, [_P, _I64, _P, _P]),
+    "svtgpu_ewise": (_INT, [_P, _INT, _P, _INT, _I64, _INT, _INT,
+                            _c.POINTER(_P), _c.POINTER(_INT)]),
 }
+
+# element-wise opcodes (SVTGPU_EW_*) and warning bits
+EW_OPCODES = {"*": 1, "/": 2, "abs": 11, "sign": 12, "sqrt": 13, "floor": 14,
+              "ceiling": 15, "trunc": 16, "log1p": 17, "expm1": 18}
+EW_WARN_INT_OVERFLOW, EW_WARN_NAN = 1, 2
+EW_WARNINGS = ((EW_WARN_INT_OVERFLOW, "NAs produced by integer overflow"),
+               (EW_WARN_NAN, "NaNs produced"))
 
 _lib = None
 

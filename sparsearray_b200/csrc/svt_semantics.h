@@ -1,9 +1,10 @@
 /* svt_semantics.h -- result composition rules of the reference, shared by the
  * CUDA kernels (device) and by tests/semantics_host.cpp (host build of the
  * very same functions, so the NA/NaN/zero-background logic can be checked on
- * a machine without a GPU).  No loops over data here: the kernels reduce a
- * leaf (or a row) to a small "partial" and these functions turn a partial
- * into the value the reference would have produced.
+ * a machine without a GPU).  No loops over data here (except the check of an
+ * element-wise operand, done once on the host): the kernels reduce a leaf (or
+ * a row) to a small "partial" and these functions turn a partial into the
+ * value the reference would have produced.
  *
  * Reference: src/Rvector_summarization.c (per-type loops :177-734, lacunar
  * :742-825, post-processing :1078-1177), src/SparseArray_summarization.c
@@ -16,6 +17,7 @@
 #define SVT_SEMANTICS_H
 
 #include <stdint.h>
+#include <stdio.h>
 #include <string.h>
 #include <math.h>
 #ifndef __cplusplus
@@ -586,6 +588,277 @@ SVT_HD double svt_dot_finalize(int is_double, double s, int leaf_flag,
 	if (hits_nonfinite < (int64_t) ci.n_nonfinite)
 		return svt_nan();
 	return svt_clean_nan(s);
+}
+
+/* ------------------------------------------------------------------------
+ * Element-wise operations that map the implicit zero to zero (svtgpu_ewise)
+ *
+ * Base R's dense semantics (src/main/arithmetic.c: R_integer_times(),
+ * real_binary(), math1(), do_abs()) restated for one stored value.  The glue
+ * calls the checks on the host before any device work; the kernels call the
+ * value rules; the result type is decided here once for both.
+ */
+
+/* refusal codes of svt_ew_check() */
+#define SVT_EW_OK           0
+#define SVT_EW_BAD_OPCODE   1  /* not an operation that keeps zeros at zero */
+#define SVT_EW_LEFT_DIV     2  /* v / x */
+#define SVT_EW_BAD_X_TYPE   3
+#define SVT_EW_BAD_V_TYPE   4
+#define SVT_EW_BAD_MARGIN   5
+#define SVT_EW_BAD_LENGTH   6
+#define SVT_EW_BAD_VALUE    7  /* *bad = 0-based index into the operand */
+
+/* bits OR-ed by the value rules (the first two are svtgpu_ewise's *warn) */
+#define SVT_EW_DROPPED      4  /* a computed value compares equal to 0 */
+
+SVT_HD int svt_ew_is_arith(int op)
+{
+	return op == SVTGPU_EW_MUL || op == SVTGPU_EW_DIV;
+}
+
+SVT_HD int svt_ew_is_math(int op)
+{
+	return op >= SVTGPU_EW_ABS && op <= SVTGPU_EW_EXPM1;
+}
+
+SVT_HD int svt_ew_streq(const char *a, const char *b)
+{
+	while (*a != '\0' && *a == *b) {
+		a++;
+		b++;
+	}
+	return *a == *b;
+}
+
+/* "*" / "/" -> opcode; any other name (the rest of R's Arith group) -> 0 */
+SVT_HD int svt_ew_arith_opcode(const char *name)
+{
+	if (svt_ew_streq(name, "*")) return SVTGPU_EW_MUL;
+	if (svt_ew_streq(name, "/")) return SVTGPU_EW_DIV;
+	return 0;
+}
+
+/* the Math-group functions with f(0) == 0 -> opcode; others -> 0 */
+SVT_HD const char *svt_ew_opname(int op)
+{
+	switch (op) {
+	    case SVTGPU_EW_MUL:     return "*";
+	    case SVTGPU_EW_DIV:     return "/";
+	    case SVTGPU_EW_ABS:     return "abs";
+	    case SVTGPU_EW_SIGN:    return "sign";
+	    case SVTGPU_EW_SQRT:    return "sqrt";
+	    case SVTGPU_EW_FLOOR:   return "floor";
+	    case SVTGPU_EW_CEILING: return "ceiling";
+	    case SVTGPU_EW_TRUNC:   return "trunc";
+	    case SVTGPU_EW_LOG1P:   return "log1p";
+	    case SVTGPU_EW_EXPM1:   return "expm1";
+	}
+	return "?";
+}
+
+SVT_HD int svt_ew_math_opcode(const char *name)
+{
+	for (int op = SVTGPU_EW_ABS; op <= SVTGPU_EW_EXPM1; op++)
+		if (svt_ew_streq(name, svt_ew_opname(op)))
+			return op;
+	return 0;
+}
+
+SVT_HD int svt_ew_type_ok(int t)
+{
+	return t == SVTGPU_LGL || t == SVTGPU_INT || t == SVTGPU_DOUBLE;
+}
+
+/* Type of the result (arithmetic.c): "/" is always double; "*" is integer
+ * when neither side is double; Math is double except abs() of integer or
+ * logical input (do_abs()). */
+SVT_HD int svt_ew_result_type(int op, int x_type, int v_type)
+{
+	if (op == SVTGPU_EW_MUL)
+		return (x_type != SVTGPU_DOUBLE && v_type != SVTGPU_DOUBLE)
+			? SVTGPU_INT : SVTGPU_DOUBLE;
+	if (op == SVTGPU_EW_ABS && x_type != SVTGPU_DOUBLE)
+		return SVTGPU_INT;
+	return SVTGPU_DOUBLE;
+}
+
+/* Would f(0) stay 0 for every element of the operand?  Arith ops only.
+ *   margin 0: v is a scalar; 1: v[i] for row i (R's recycling of `x op v`
+ *   with length(v) == nrow, any number of dimensions); 2: v[j] for column j
+ *   (`sweep(x, 2, v, op)`, 2-D only; nleaf columns).
+ * Returns SVT_EW_OK or a refusal code; *bad receives the offending element
+ * for SVT_EW_BAD_VALUE. */
+SVT_HD int svt_ew_check(int op, int x_type, int v_type, int64_t v_len,
+			int margin, int v_on_left, int ndim, int64_t nrow,
+			int64_t nleaf, const void *v, int64_t *bad)
+{
+	*bad = -1;
+	if (!svt_ew_type_ok(x_type))
+		return SVT_EW_BAD_X_TYPE;
+	if (svt_ew_is_math(op))
+		return SVT_EW_OK;
+	if (!svt_ew_is_arith(op))
+		return SVT_EW_BAD_OPCODE;
+	if (op == SVTGPU_EW_DIV && v_on_left)
+		return SVT_EW_LEFT_DIV;
+	if (!svt_ew_type_ok(v_type))
+		return SVT_EW_BAD_V_TYPE;
+	if (margin < 0 || margin > 2 || (margin == 2 && ndim != 2))
+		return SVT_EW_BAD_MARGIN;
+	const int64_t want = margin == 0 ? 1 : margin == 1 ? nrow : nleaf;
+	if (v_len != want)
+		return SVT_EW_BAD_LENGTH;
+	for (int64_t i = 0; i < v_len; i++) {
+		int ok;
+		if (v_type == SVTGPU_DOUBLE) {
+			const double d = ((const double *) v)[i];
+			/* 0 * Inf is NaN, 0 * NA is NA; 0 / 0 is NaN, 0 / NA
+			   is NA; 0 / Inf is 0 */
+			ok = op == SVTGPU_EW_MUL ? svt_isfinite(d)
+						 : !svt_isnan(d) && d != 0.0;
+		} else {
+			const int32_t k = ((const int32_t *) v)[i];
+			ok = k != SVT_NA_INT && (op == SVTGPU_EW_MUL || k != 0);
+		}
+		if (!ok) {
+			*bad = i;
+			return SVT_EW_BAD_VALUE;
+		}
+	}
+	return SVT_EW_OK;
+}
+
+static inline const char *svt_ew_value_name(int v_type, const void *v,
+					    int64_t i)
+{
+	if (v_type != SVTGPU_DOUBLE)
+		return ((const int32_t *) v)[i] == SVT_NA_INT ? "NA" : "0";
+	const double d = ((const double *) v)[i];
+	if (svt_is_na_real(d)) return "NA";
+	if (svt_isnan(d)) return "NaN";
+	if (d == svt_posinf()) return "Inf";
+	if (d == svt_neginf()) return "-Inf";
+	return "0";
+}
+
+/* The R error message of a refusal (host only).  `opname` is the name the
+ * caller was given (it may be an operator svt_ew_check() does not know). */
+static inline void svt_ew_refusal_message(int code, const char *opname,
+					  int is_math, int op, int v_type, const void *v,
+					  int64_t v_len, int margin,
+					  int64_t nrow, int64_t nleaf,
+					  int64_t bad, char *buf, size_t len)
+{
+	switch (code) {
+	    case SVT_EW_BAD_OPCODE:
+		if (is_math)
+			snprintf(buf, len, "Math function \"%s\" is not supported "
+				 "on a SparseArray on the GPU path: it does not "
+				 "map zero to zero (supported: abs, sign, sqrt, "
+				 "floor, ceiling, trunc, log1p, expm1)", opname);
+		else
+			snprintf(buf, len, "Arith operator \"%s\" is not "
+				 "supported on a SparseArray on the GPU path: it "
+				 "would turn the implicit zeros into nonzero "
+				 "values (supported: \"*\" and \"/\")", opname);
+		return;
+	    case SVT_EW_LEFT_DIV:
+		snprintf(buf, len, "operator \"/\" with the SparseArray on the "
+			 "right is not supported: the implicit zeros would "
+			 "become Inf, NA or NaN");
+		return;
+	    case SVT_EW_BAD_X_TYPE:
+		snprintf(buf, len, "\"%s\": only logical, integer and double "
+			 "SparseArray objects are supported on the GPU path",
+			 opname);
+		return;
+	    case SVT_EW_BAD_V_TYPE:
+		snprintf(buf, len, "operator \"%s\": the operand must be a "
+			 "logical, integer or double vector", opname);
+		return;
+	    case SVT_EW_BAD_MARGIN:
+		snprintf(buf, len, "operator \"%s\": MARGIN must be 0 (a scalar), "
+			 "1 (along the rows) or 2 (along the columns of a "
+			 "2-D object)", opname);
+		return;
+	    case SVT_EW_BAD_LENGTH:
+		if (margin == 0)
+			snprintf(buf, len, "operator \"%s\": the operand has "
+				 "length %lld, a scalar operand must have length "
+				 "1", opname, (long long) v_len);
+		else
+			snprintf(buf, len, "operator \"%s\": the operand has "
+				 "length %lld, it must have length %s = %lld",
+				 opname, (long long) v_len,
+				 margin == 1 ? "nrow(x)" : "ncol(x)",
+				 (long long) (margin == 1 ? nrow : nleaf));
+		return;
+	    case SVT_EW_BAD_VALUE:
+		snprintf(buf, len, "operator \"%s\": element %lld of the operand "
+			 "is %s, so the implicit zeros of the result would be "
+			 "%s", opname, (long long) bad + 1,
+			 svt_ew_value_name(v_type, v, bad),
+			 op == SVTGPU_EW_MUL ? "NaN or NA (0 * Inf, 0 * NA)"
+					     : "NaN or NA (0 / 0, 0 / NA)");
+		return;
+	}
+	snprintf(buf, len, "operator \"%s\": refused (code %d)", opname, code);
+}
+
+/* Integer result: `x * v` of two integers (R_integer_times(): the product
+ * in 64 bits, NA_integer_ with the overflow warning when it leaves the int
+ * range or equals INT_MIN) and abs() of an integer.  v is never NA. */
+SVT_HD int32_t svt_ew_int(int op, int32_t x, int32_t v, uint32_t *fl)
+{
+	if (x == SVT_NA_INT)
+		return SVT_NA_INT;
+	int64_t z = op == SVTGPU_EW_MUL ? (int64_t) x * (int64_t) v
+					: (x < 0 ? -(int64_t) x : (int64_t) x);
+	if (z > INT32_MAX || z <= INT32_MIN) {
+		*fl |= SVTGPU_EW_WARN_INT_OVERFLOW;
+		return SVT_NA_INT;
+	}
+	if (z == 0)
+		*fl |= SVT_EW_DROPPED;
+	return (int32_t) z;
+}
+
+/* Double result.  x_na: the input is NA (integer NA_integer_ or R_IsNA()).
+ * NA stays NA_real_ and any other NaN keeps its own bits (math1(): "keep NA
+ * vs NaN distinction"; for "*" and "/" the x86 FPU returns the NaN operand).
+ * A NaN produced from a non-NaN value is the canonical quiet NaN; from a
+ * Math function it sets the "NaNs produced" warning (math1()), from "*" or
+ * "/" (Inf * 0, Inf / Inf) it does not (real_binary()). */
+SVT_HD double svt_ew_dbl(int op, double x, int x_na, double v, uint32_t *fl)
+{
+	if (x_na)
+		return svt_na_real();
+	if (svt_isnan(x))
+		return x;
+	double r;
+	switch (op) {
+	    case SVTGPU_EW_MUL:     r = x * v; break;
+	    case SVTGPU_EW_DIV:     r = x / v; break;
+	    case SVTGPU_EW_ABS:     r = fabs(x); break;
+	    case SVTGPU_EW_SIGN:    r = x > 0.0 ? 1.0 : (x < 0.0 ? -1.0 : 0.0);
+				    break;
+	    case SVTGPU_EW_SQRT:    r = sqrt(x); break;
+	    case SVTGPU_EW_FLOOR:   r = floor(x); break;
+	    case SVTGPU_EW_CEILING: r = ceil(x); break;
+	    case SVTGPU_EW_TRUNC:   r = trunc(x); break;
+	    case SVTGPU_EW_LOG1P:   r = log1p(x); break;
+	    case SVTGPU_EW_EXPM1:   r = expm1(x); break;
+	    default:                r = svt_nan(); break;
+	}
+	if (svt_isnan(r)) {
+		if (svt_ew_is_math(op))
+			*fl |= SVTGPU_EW_WARN_NAN;
+		return svt_nan();
+	}
+	if (r == 0.0)
+		*fl |= SVT_EW_DROPPED;
+	return r;
 }
 
 #endif  /* SVT_SEMANTICS_H */

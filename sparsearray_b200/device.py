@@ -180,6 +180,65 @@ class DeviceSVT:
         except Exception:
             pass
 
+    # -- element-wise operations (new shard, no collective) ------------
+    def ewise(self, op, operand=None, margin=0, operand_on_left=False):
+        """x * v, v * x, x / v (op "*" / "/") or a Math function ("abs",
+        "sign", "sqrt", "floor", "ceiling", "trunc", "log1p", "expm1") as a
+        new owning DeviceSVT with the same columns; see svtgpu_ewise() in
+        include/svtgpu.h.  margin 2 takes the per-column vector of the whole
+        matrix (length nleaf_total, sliced to this shard's columns) or this
+        shard's slice.  The result's `warnings` lists R's warnings."""
+        code = N.EW_OPCODES.get(op)
+        if code is None:
+            raise ValueError("unsupported element-wise operation %r" % (op,))
+        vp, vt, vlen = None, 0, 0
+        keep = None
+        if code in (N.EW_OPCODES["*"], N.EW_OPCODES["/"]):
+            a = np.asarray(operand).reshape(-1)
+            if margin == 2 and a.size == self.nleaf_total and \
+                    self.nleaf != self.nleaf_total:
+                a = a[self.leaf0:self.leaf0 + self.nleaf]
+            if a.dtype.kind == "b":
+                keep, vt = np.ascontiguousarray(a, dtype=np.int32), N.LGL
+            elif a.dtype.kind in "iu":
+                keep, vt = np.ascontiguousarray(a, dtype=np.int32), N.INT
+            else:
+                keep, vt = np.ascontiguousarray(a, dtype=np.float64), N.DOUBLE
+            vp, vlen = keep.ctypes.data_as(ctypes.c_void_p), keep.size
+        h = ctypes.c_void_p()
+        warn = ctypes.c_int(0)
+        N.check(N.lib().svtgpu_ewise(self._h, code, vp, vt, vlen, int(margin),
+                                     int(operand_on_left), ctypes.byref(h),
+                                     ctypes.byref(warn)))
+        nnz, vtype = ctypes.c_int64(0), ctypes.c_int(0)
+        N.check(N.lib().svtgpu_matrix_info(h, None, None, ctypes.byref(nnz),
+                                           ctypes.byref(vtype), None))
+        type_ = {N.INT: "integer", N.DOUBLE: "double"}[vtype.value]
+        out = DeviceSVT(self.nrow, self.nleaf, nnz.value, type_, None, None,
+                        None, leaf0=self.leaf0, nleaf_total=self.nleaf_total,
+                        handle=h, owns_handle=True)
+        out.warnings = [msg for bit, msg in N.EW_WARNINGS if warn.value & bit]
+        return out
+
+    def download(self):
+        """(leaf_ptr, offs, vals) of the shard on the host (vals None when
+        the shard stores no values)."""
+        L = N.lib()
+        flags = ctypes.c_int(0)
+        N.check(L.svtgpu_matrix_info(self._h, None, None, None, None,
+                                     ctypes.byref(flags)))
+        ptr = np.zeros(self.nleaf + 1, dtype=np.int64)
+        offs = np.zeros(self.nnz, dtype=np.int32)
+        vals = None
+        if flags.value & N.HAS_VALS:
+            vals = np.zeros(self.nnz, dtype=np.float64
+                            if self.val_type == "double" else np.int32)
+        N.check(L.svtgpu_matrix_download(
+            self._h, ptr.ctypes.data_as(ctypes.c_void_p),
+            offs.ctypes.data_as(ctypes.c_void_p),
+            None if vals is None else vals.ctypes.data_as(ctypes.c_void_p)))
+        return ptr, offs, vals
+
     # -- column statistics (no collective) ----------------------------
     def colstats(self, op, na_rm=False, center=None, out=None, warn=None):
         """One value per local column, left on the device."""

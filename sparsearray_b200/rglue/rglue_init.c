@@ -66,6 +66,8 @@ static const R_CallMethodDef callMethods[] = {
 	CALLMETHOD_DEF(C_svtgpu_release, 1),
 	CALLMETHOD_DEF(C_svtgpu_from_CSC, 5),
 	CALLMETHOD_DEF(C_svtgpu_to_CSC, 2),
+	CALLMETHOD_DEF(C_svtgpu_Arith_SVT, 7),
+	CALLMETHOD_DEF(C_svtgpu_Math_SVT, 4),
 	CALLMETHOD_DEF(C_svtgpu_set_cache, 1),
 	CALLMETHOD_DEF(C_svtgpu_cache_stats, 0),
 	{NULL, NULL, 0}

@@ -209,6 +209,21 @@ class SVT_SparseArray:
         except Exception:
             pass
 
+    # -- Arith with R's recycling (x op v, v op x); see Arith() ------------
+    __array_ufunc__ = None   # `ndarray * x` defers to x instead of broadcasting
+
+    def __mul__(self, other):
+        return Arith(self, "*", other)
+
+    def __rmul__(self, other):
+        return Arith(other, "*", self)
+
+    def __truediv__(self, other):
+        return Arith(self, "/", other)
+
+    def __rtruediv__(self, other):
+        return Arith(other, "/", self)   # refused: v / x
+
 
 class ResidentSVT(SVT_SparseArray):
     """An SVT_SparseArray whose SVT already lives in HBM: `r_SVT` is the
@@ -276,6 +291,116 @@ def from_csc(dim, indptr, data, indices, indices_are_1based=False):
     r.dimnames = [None] * len(r.dim)
     r._robjs = {"dim": rshim.integer(list(r.dim)), "dimnames": None,
                 "type": rshim.string(r.type), "SVT": rshim.RObj(ans)}
+    return r
+
+
+def _resident_like(x, handle, type_):
+    """A ResidentSVT around a new handle, with x's dim and dimnames (built
+    the way from_csc() builds one)."""
+    r = ResidentSVT.__new__(ResidentSVT)
+    r.dim, r.type = tuple(x.dim), type_
+    r.ptr = r.offs = r.vals = r.lacunar = None
+    r.dimnames = [None if d is None else list(d) for d in x.dimnames]
+    r._robjs = {"dim": rshim.integer(list(r.dim)),
+                "dimnames": _dimnames_robj(_simplify_NULL_dimnames(
+                    r.dimnames)),
+                "type": rshim.string(r.type), "SVT": handle}
+    return r
+
+
+def _operand(v):
+    """A numeric vector / scalar as an R vector: bool -> logical, integers ->
+    integer (values outside the int range -> double), floats -> double."""
+    a = np.asarray(v).reshape(-1)
+    if a.dtype.kind == "b":
+        return rshim.wrap(a.astype(np.int32), rshim.LGLSXP)
+    if a.dtype.kind in "iu":
+        if a.size == 0 or (a.min() >= -2**31 and a.max() <= 2**31 - 1):
+            return rshim.wrap(a.astype(np.int32), rshim.INTSXP)
+        return rshim.wrap(a.astype(np.float64), rshim.REALSXP)
+    if a.dtype.kind == "f":
+        return rshim.wrap(a.astype(np.float64), rshim.REALSXP)
+    raise TypeError("non-numeric argument to binary operator")
+
+
+def _ewise_result(ans, x):
+    import ctypes
+    elts = ctypes.cast(ans.contents.data, ctypes.POINTER(rshim.SEXP))
+    type_ = rshim.strings(elts[1])[0]
+    # a pointer of its own: elts[0] aliases the list slot cleared below
+    handle = rshim.RObj(ctypes.cast(
+        ctypes.c_void_p(ctypes.cast(elts[0], ctypes.c_void_p).value),
+        rshim.SEXP))
+    # detach the handle: releasing the list must not run its finalizer
+    rshim.lib().SET_VECTOR_ELT(ans, 0, rshim.nil())
+    rshim.lib().rshim_release_tree(ans)
+    return _resident_like(x, handle, type_)
+
+
+def _arith_call(x, op, y, margin, y_on_left):
+    if not isinstance(op, str):
+        raise TypeError("'op' must be a single string")
+    yv = _operand(y)
+    temps = [yv, rshim.string(op), rshim.integer([margin]),
+             rshim.logical([int(y_on_left)])]
+    try:
+        ans, warns = rcall.SparseArray_Call(
+            "C_svtgpu_Arith_SVT", x.r_dim, x.r_type, x.r_SVT, temps[1], yv,
+            temps[2], temps[3])
+    finally:
+        for t in temps:
+            t.release()
+    r = _ewise_result(ans, x)
+    r.warnings = warns
+    return r
+
+
+def Arith(e1, op, e2):
+    """`e1 op e2` for op "*" or "/" where one side is an SVT_SparseArray and
+    the other a numeric scalar or a vector of length nrow(x) (recycled along
+    the first dimension, as R does).  Any other operand length is refused, as
+    is `v / x` and every operation that would turn the implicit zeros into
+    something else (`x * Inf`, `x * NA`, `x / 0`, "+", ...).  Served on the
+    device: returns a new ResidentSVT (result type as in base R), with
+    `.warnings` holding R's warnings."""
+    if isinstance(e1, SVT_SparseArray):
+        x, y, on_left = e1, e2, False
+    elif isinstance(e2, SVT_SparseArray):
+        x, y, on_left = e2, e1, True
+    else:
+        raise TypeError("one operand must be an SVT_SparseArray")
+    n = np.asarray(y).size
+    return _arith_call(x, op, y, 0 if n == 1 else 1, on_left)
+
+
+def sweep(x, MARGIN, STATS, FUN="-"):
+    """sweep(x, MARGIN, STATS, FUN) for FUN "*" or "/": STATS[i] applied to
+    row i (MARGIN = 1) or STATS[j] to column j of a matrix (MARGIN = 2), as
+    `t(t(x) / sf)`.  FUN defaults to "-" as in R, which is refused (it would
+    fill the implicit zeros)."""
+    if not isinstance(x, SVT_SparseArray):
+        raise TypeError("'x' must be an SVT_SparseArray")
+    if MARGIN not in (1, 2):
+        _wmsg_stop("'MARGIN' must be 1 or 2")
+    return _arith_call(x, FUN, STATS, int(MARGIN), False)
+
+
+def Math(x, op):
+    """op(x) for the Math functions that map 0 to 0: abs, sign, sqrt, floor,
+    ceiling, trunc, log1p, expm1 (any other name is refused).  Result type
+    double, except abs() of integer / logical input; NA and NaN keep their
+    kind; `.warnings` holds "NaNs produced" when one was made.  Returns a new
+    ResidentSVT."""
+    if not isinstance(x, SVT_SparseArray):
+        raise TypeError("'x' must be an SVT_SparseArray")
+    t = rshim.string(op)
+    try:
+        ans, warns = rcall.SparseArray_Call("C_svtgpu_Math_SVT", x.r_dim,
+                                            x.r_type, x.r_SVT, t)
+    finally:
+        t.release()
+    r = _ewise_result(ans, x)
+    r.warnings = warns
     return r
 
 

@@ -97,6 +97,25 @@ def poisson_csc(nrow, nleaf, density, seed=0, na_rate=0.0, leaf0=0,
     return ptr, offs, vals
 
 
+def poisson_row(nrow, nleaf, i, density, seed=0, na_rate=0.0, leaf0=0):
+    """Row i of the matrix poisson_csc() makes, evaluated on its own (cell
+    (i, l) depends only on l * nrow + i): (leaves, values, is_na), leaves
+    relative to leaf0 and ascending, values int64 (those under is_na are
+    the draws that became NA).  The values of a lacunar matrix are ignored."""
+    nz_thr, vthr = poisson_thresholds(density)
+    na_thr = np.uint64(na_threshold(na_rate))
+    l = np.arange(leaf0, leaf0 + nleaf, dtype=np.uint64)
+    with np.errstate(over="ignore"):
+        h = mix64(np.uint64(seed) +
+                  (l * np.uint64(nrow) + np.uint64(i) + np.uint64(1)) * GOLDEN)
+        cols = np.flatnonzero((h >> np.uint64(32)) < np.uint64(nz_thr))
+        h2 = mix64(h[cols] ^ SALT2)
+        v = 1 + np.searchsorted(vthr.astype(np.uint64), h2 >> np.uint64(32),
+                                side="right")
+        is_na = (h2 & np.uint64(0xFFFFFFFF)) < na_thr
+    return cols, v.astype(np.int64), is_na
+
+
 def poisson_svt(nrow, ncol, density, seed=0, na_rate=0.0, type="integer",
                 lacunar=False):
     ptr, offs, vals = poisson_csc(nrow, ncol, density, seed, na_rate, 0, type,

@@ -123,7 +123,9 @@ int svtgpu_matrix_create(svtgpu_matrix **m, int64_t nrow, int64_t nleaf,
 			 int64_t nnz, int val_type, int flags);
 /* Wrap device arrays owned by the caller (no copies, not freed by free()).
  * d_offs / d_vals must be 16-byte aligned and readable for 64 elements past
- * nnz (the optional bulk-copy kernels round their reads up to 16 bytes). */
+ * nnz (the optional bulk-copy kernels round their reads up to 16 bytes).
+ * The arrays must not change while they are wrapped: the handle caches what
+ * it learns from them (max |x|, the row-tile tables, a compact copy). */
 int svtgpu_matrix_wrap_device(svtgpu_matrix **m, int64_t nrow, int64_t nleaf,
 			      int64_t nnz, int val_type,
 			      const int64_t *d_leaf_ptr, const int32_t *d_offs,
@@ -194,6 +196,13 @@ int svtgpu_matrix_set_leaf_base(svtgpu_matrix *m, int64_t leaf_base);
 int svtgpu_matrix_info(const svtgpu_matrix *m, int64_t *nrow, int64_t *nleaf,
 		       int64_t *nnz, int *val_type, int *flags);
 int svtgpu_matrix_timings(const svtgpu_matrix *m, svtgpu_timings *t);
+/* Device bytes held by the matrix's compact copy of its entries (0 = none).
+ * Integer and logical matrices whose values lie in [-127, 127] get int8
+ * values (and uint16 row offsets when nrow <= 65536) on the second column-sum
+ * or row-sum / row-moment call on the handle; those statistics then read the
+ * narrow arrays.  The copy is freed with the matrix and dropped when its
+ * entries are rewritten (upload, svtgpu_matrix_fold_rows). */
+int svtgpu_matrix_compact_bytes(const svtgpu_matrix *m, int64_t *bytes);
 
 /* ---- column statistics ----
  * One result per group of `group` consecutive leaves (group = 1 for a matrix

@@ -69,6 +69,7 @@ SIGNATURES = {
                                   _c.POINTER(_I64), _c.POINTER(_INT),
                                   _c.POINTER(_INT)]),
     "svtgpu_matrix_timings": (_INT, [_P, _c.POINTER(Timings)]),
+    "svtgpu_matrix_compact_bytes": (_INT, [_P, _c.POINTER(_I64)]),
     "svtgpu_colstats": (_INT, [_P, _INT, _INT, _DBL, _I64, _P,
                                _c.POINTER(_INT)]),
     "svtgpu_colstats_dev": (_INT, [_P, _INT, _INT, _DBL, _I64, _P, _P, _P]),

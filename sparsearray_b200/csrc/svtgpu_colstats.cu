@@ -527,6 +527,90 @@ colstats_direct(ColParams P)
 }
 
 /* ------------------------------------------------------------------------
+ * colstats_sum_i8: the integer SUM class (colSums, colMeans) over the compact
+ * int8 values (svtgpu_internal.h).  A warp per segment, 16-byte loads over
+ * the aligned middle with up to four per lane in flight, single bytes at the
+ * ends.  Per 32-bit word __dp4a gives the signed byte sum, in which every NA
+ * byte (-128) counts -128, and __vcmpeq4 marks the NA bytes (0xFF each), so
+ * sum = dp4a + 128 #NA exactly: the partial equals the wide kernel's.
+ */
+__device__ __forceinline__ void sum_i8_word(uint32_t w, int &s, int &na_bits)
+{
+	s = __dp4a((int) w, 0x01010101, s);
+	na_bits += __popc(__vcmpeq4(w, 0x80808080u));
+}
+
+#define SUM_I8_BLOCKS_PER_SM 6   /* 40 registers: four 16-byte loads in flight */
+__global__ void __launch_bounds__(256, SUM_I8_BLOCKS_PER_SM)
+colstats_sum_i8(ColParams P, const int8_t *__restrict__ v8)
+{
+	const int lane = threadIdx.x & 31;
+	const int64_t warps = ((int64_t) gridDim.x * blockDim.x) >> 5;
+	const int64_t gw = ((int64_t) blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+	/* a C2 leaf is ~2.3 KB: its bounds are requested a segment ahead */
+	int64_t nstart = 0, nend = 0;
+	if (gw < P.nseg) {
+		nstart = P.leaf_ptr[gw * P.group];
+		nend = P.leaf_ptr[(gw + 1) * P.group];
+	}
+	for (int64_t seg = gw; seg < P.nseg; seg += warps) {
+		const int64_t start = nstart, end = nend;
+		if (seg + warps < P.nseg) {
+			nstart = P.leaf_ptr[(seg + warps) * P.group];
+			nend = P.leaf_ptr[(seg + warps + 1) * P.group];
+		}
+		long long sum = 0;
+		int na_bits = 0;   /* 8 per NA */
+		const int64_t a16 = (start + 15) & ~(int64_t) 15;
+		const int64_t b16 = end & ~(int64_t) 15;
+		int64_t lo = start, hi = end;   /* bytes left to single lanes */
+		if (a16 < b16) {
+			const uint4 *q = (const uint4 *) (v8 + a16);
+			const int nv = (int) ((b16 - a16) >> 4);
+			for (int i = lane; i < nv; i += 128) {
+				uint4 u[4];
+#pragma unroll
+				for (int k = 0; k < 4; k++)
+					u[k] = i + 32 * k < nv ? __ldcs(q + i + 32 * k)
+							       : make_uint4(0, 0, 0, 0);
+				int s = 0;
+#pragma unroll
+				for (int k = 0; k < 4; k++) {
+					sum_i8_word(u[k].x, s, na_bits);
+					sum_i8_word(u[k].y, s, na_bits);
+					sum_i8_word(u[k].z, s, na_bits);
+					sum_i8_word(u[k].w, s, na_bits);
+				}
+				sum += s;
+			}
+			/* < 16 bytes at either end */
+			if (start + lane < a16) {
+				const int x = v8[start + lane];
+				sum += x;
+				na_bits += x == SVT_COMPACT_NA_I8 ? 8 : 0;
+			}
+			lo = b16;
+		}
+		for (int64_t e = lo + lane; e < hi; e += 32) {
+			const int x = v8[e];
+			sum += x;
+			na_bits += x == SVT_COMPACT_NA_I8 ? 8 : 0;
+		}
+		const long long n_na = svt_warp_sum((long long) na_bits) >> 3;
+		sum = svt_warp_sum(sum) + 128 * n_na;
+		if (lane == 0) {
+			SvtColPartial part;
+			svt_col_partial_init(&part);
+			part.nz = end - start;
+			part.n_na = n_na;
+			part.sum = (double) sum;
+			store_result(P, seg, svt_col_finalize(P.opcode, P.is_double,
+					P.narm, P.seg_len, P.center, &part));
+		}
+	}
+}
+
+/* ------------------------------------------------------------------------
  * colstats_tma
  */
 
@@ -851,7 +935,7 @@ int launch_typed(const ColParams &P, int cc, bool use_tma, int avg_seg_bytes,
 
 }  /* namespace */
 
-int svtgpu_launch_colstats(const svtgpu_matrix *m, int opcode, int narm,
+int svtgpu_launch_colstats(svtgpu_matrix *m, int opcode, int narm,
 			   double center, int64_t group, void *d_out,
 			   int32_t *d_warn, cudaStream_t stream)
 {
@@ -900,6 +984,21 @@ int svtgpu_launch_colstats(const svtgpu_matrix *m, int opcode, int narm,
 		return SVTGPU_OK;
 	}
 	const int cc = col_class_of(opcode);
+	if (cc == CC_SUM && !P.is_double) {
+		SVT_CHECK(svt_ensure_compact(m, stream));
+		if (m->d_vals8 != NULL) {
+			int64_t blocks = (P.nseg + 7) / 8;
+			const int64_t cap = (int64_t) svtgpu_sm_count() *
+					    SUM_I8_BLOCKS_PER_SM;
+			if (blocks > cap)
+				blocks = cap;
+			colstats_sum_i8<<<(unsigned) blocks, 256, 0, stream>>>(
+				P, m->d_vals8);
+			SVT_CUDA(cudaGetLastError());
+			svtgpu_count_launch(1);
+			return SVTGPU_OK;
+		}
+	}
 	const char *impl = svtgpu_env("SVTGPU_COLSTATS_IMPL", "direct");
 	bool use_tma = strcmp(impl, "tma") == 0 &&
 		       (((uintptr_t) m->d_vals) & 15) == 0;

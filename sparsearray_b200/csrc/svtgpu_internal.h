@@ -58,9 +58,43 @@ struct svtgpu_matrix {
 	int64_t leaf_base;   /* global index of leaf 0 when m is a column shard */
 	struct svtgpu_matrix *transposed;   /* cached t(m), owned by m */
 	int transpose_failed;
+	/* compact copy of the entries, owned by m (see svt_ensure_compact) */
+	uint16_t *d_offs16;  /* nnz + SVT_COMPACT_PAD, or NULL */
+	int8_t *d_vals8;     /* nnz + SVT_COMPACT_PAD, or NULL */
+	int compact_state;   /* SVT_COMPACT_NONE / _BUILT / _INELIGIBLE */
+	int compact_uses;    /* eligible statistic calls seen while NONE */
 
 	svtgpu_timings tm;
 };
+
+/* ---- compact copy ----
+ * The hot statistics of small-count integer matrices are bound by the bytes
+ * they read, and 4-byte offsets and values mostly carry padding.  A matrix may
+ * hold a second, narrow copy of its entries beside the wide arrays:
+ *   d_vals8   int8 values; NA is SVT_COMPACT_NA_I8 (-128).  Built for integer
+ *             and logical matrices whose non-NA values all lie in [-127, 127]
+ *             (vmax_abs <= 127, so no stored value is -128).
+ *   d_offs16  uint16 row offsets.  Built for nrow <= 65536, and only beside
+ *             d_vals8: no kernel reads the offsets alone.
+ * Both are padded by SVT_COMPACT_PAD zeroed entries so that 16-byte loads
+ * past the last entry stay inside the allocation.  The copy is built on the
+ * second eligible statistic call on a handle (a handle used once never pays
+ * for it), dropped wherever the wide arrays are rewritten, and not inherited
+ * by derived matrices. */
+#define SVT_COMPACT_NA_I8 (-128)
+#define SVT_COMPACT_PAD 64
+#define SVT_COMPACT_NONE 0
+#define SVT_COMPACT_BUILT 1
+#define SVT_COMPACT_INELIGIBLE 2
+#define SVT_COMPACT_MAX_ABS 127
+#define SVT_COMPACT_MAX_NROW 65536
+
+/* Count one eligible statistic call on m and build the compact copy on the
+   second (synchronises s once).  Never fails for lack of memory: the matrix
+   is then marked ineligible and the wide arrays serve. */
+int svt_ensure_compact(svtgpu_matrix *m, cudaStream_t s);
+/* Free the compact copy (stream-ordered on s) and forget that it was decided. */
+void svt_drop_compact(svtgpu_matrix *m, cudaStream_t s);
 
 /* upper bound of |x| over the non-NA values of an integer matrix when one is
    known without a pass over the data, else -1 */
@@ -120,7 +154,7 @@ int svtgpu_ensure_split(svtgpu_matrix *m, int nstrips, int strip_rows,
 			cudaStream_t s, const int32_t **split);
 int svtgpu_ensure_transpose(svtgpu_matrix *m, cudaStream_t s,
 			    svtgpu_matrix **out);
-int svtgpu_launch_colstats(const svtgpu_matrix *m, int opcode, int narm,
+int svtgpu_launch_colstats(svtgpu_matrix *m, int opcode, int narm,
 			   double center, int64_t group, void *d_out,
 			   int32_t *d_warn, cudaStream_t stream);
 int svtgpu_launch_row_accumulate(svtgpu_matrix *m, int opcode, int narm,

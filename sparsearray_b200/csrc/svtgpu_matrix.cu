@@ -538,6 +538,7 @@ extern "C" int svtgpu_matrix_free(svtgpu_matrix *m)
 	for (int i = 0; i < SVTGPU_NSPLIT; i++)
 		if (m->d_split[i]) svt_free_async(m->d_split[i], 0);
 	if (m->d_hist_tiles) svt_free_async(m->d_hist_tiles, 0);
+	svt_drop_compact(m, 0);
 	cudaDeviceSynchronize();
 	if (m->up_begin) cudaEventDestroy(m->up_begin);
 	if (m->up_end) cudaEventDestroy(m->up_end);
@@ -647,6 +648,9 @@ extern "C" int svtgpu_matrix_fold_rows(svtgpu_matrix *m, int64_t fold)
 		svt_free_async(m->d_hist_tiles, s);
 	m->d_hist_tiles = NULL;
 	m->hist_tile = 0;
+	/* the compact offsets hold the old rows (and nrow may now exceed
+	   what 16 bits can hold) */
+	svt_drop_compact(m, s);
 	return SVTGPU_OK;
 }
 
@@ -690,6 +694,8 @@ extern "C" int svtgpu_matrix_timings(const svtgpu_matrix *m, svtgpu_timings *t)
 
 static int upload_begin(svtgpu_matrix *m)
 {
+	/* the entries are about to be rewritten */
+	svt_drop_compact(m, m->up_stream);
 	if (!m->up_begun) {
 		SVT_CUDA(cudaEventRecord(m->up_begin, m->up_stream));
 		m->up_begun = 1;
@@ -961,6 +967,124 @@ extern "C" int svtgpu_matrix_commit_packed(svtgpu_matrix *m, int64_t dst,
 	g_pool.busy[s] = 1;
 	m->stage_busy[s] = 1;
 	m->stage_cur = -1;
+	return SVTGPU_OK;
+}
+
+/* ---- compact copy: narrow the wide arrays in HBM (the mirror of widen_*) ----
+ * Groups of 16 entries, cyclic over the grid: four 16-byte loads of values ->
+ * one 16-byte store, four of offsets -> two.  Unaligned wide arrays (a caller
+ * may wrap any pointer) take the scalar loop for everything. */
+__device__ __forceinline__ uint32_t narrow_byte(int32_t x)
+{
+	return x == SVT_NA_INT ? (uint32_t) (uint8_t) SVT_COMPACT_NA_I8
+			       : (uint32_t) (uint8_t) x;
+}
+
+__global__ void __launch_bounds__(256)
+narrow_compact(const int32_t *__restrict__ offs,
+	       const int32_t *__restrict__ vals, uint16_t *__restrict__ o16,
+	       int8_t *__restrict__ v8, int64_t n, int vec)
+{
+	const int64_t stride = (int64_t) gridDim.x * blockDim.x;
+	const int64_t t0 = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
+	const int64_t ng = vec ? n / 16 : 0;
+	for (int64_t g = t0; g < ng; g += stride) {
+		const int4 *qv = (const int4 *) vals + 4 * g;
+		uint32_t w[4];
+#pragma unroll
+		for (int k = 0; k < 4; k++) {
+			const int4 a = __ldcs(qv + k);
+			w[k] = narrow_byte(a.x) | (narrow_byte(a.y) << 8) |
+			       (narrow_byte(a.z) << 16) | (narrow_byte(a.w) << 24);
+		}
+		((uint4 *) v8)[g] = make_uint4(w[0], w[1], w[2], w[3]);
+		if (o16 == NULL)
+			continue;
+		const int4 *qo = (const int4 *) offs + 4 * g;
+		uint32_t h[8];
+#pragma unroll
+		for (int k = 0; k < 4; k++) {
+			const int4 a = __ldcs(qo + k);
+			h[2 * k] = ((uint32_t) a.x & 0xFFFFu) | ((uint32_t) a.y << 16);
+			h[2 * k + 1] = ((uint32_t) a.z & 0xFFFFu) |
+				       ((uint32_t) a.w << 16);
+		}
+		((uint4 *) o16)[2 * g] = make_uint4(h[0], h[1], h[2], h[3]);
+		((uint4 *) o16)[2 * g + 1] = make_uint4(h[4], h[5], h[6], h[7]);
+	}
+	for (int64_t i = ng * 16 + t0; i < n; i += stride) {
+		v8[i] = (int8_t) narrow_byte(vals[i]);
+		if (o16 != NULL)
+			o16[i] = (uint16_t) offs[i];
+	}
+}
+
+void svt_drop_compact(svtgpu_matrix *m, cudaStream_t s)
+{
+	if (m->d_offs16 != NULL)
+		svt_free_async(m->d_offs16, s);
+	if (m->d_vals8 != NULL)
+		svt_free_async(m->d_vals8, s);
+	m->d_offs16 = NULL;
+	m->d_vals8 = NULL;
+	m->compact_state = SVT_COMPACT_NONE;
+	m->compact_uses = 0;
+}
+
+int svt_ensure_compact(svtgpu_matrix *m, cudaStream_t s)
+{
+	if (m->compact_state != SVT_COMPACT_NONE)
+		return SVTGPU_OK;
+	if (svt_is_double(m->val_type) || !(m->flags & SVTGPU_HAS_VALS) ||
+	    m->nnz == 0) {
+		m->compact_state = SVT_COMPACT_INELIGIBLE;
+		return SVTGPU_OK;
+	}
+	if (++m->compact_uses < 2)
+		return SVTGPU_OK;
+	SVT_CHECK(svtgpu_ensure_absmax(m, s));
+	if (m->vmax_abs > SVT_COMPACT_MAX_ABS) {
+		m->compact_state = SVT_COMPACT_INELIGIBLE;
+		return SVTGPU_OK;
+	}
+	const bool want_offs = (m->flags & SVTGPU_HAS_OFFS) &&
+			       m->nrow <= SVT_COMPACT_MAX_NROW;
+	const size_t n = (size_t) m->nnz + SVT_COMPACT_PAD;
+	cudaError_t e = svt_malloc_async((void **) &m->d_vals8, n, s);
+	if (e == cudaSuccess && want_offs)
+		e = svt_malloc_async((void **) &m->d_offs16, 2 * n, s);
+	if (e == cudaErrorMemoryAllocation) {
+		/* the wide arrays serve as before */
+		cudaGetLastError();
+		svt_drop_compact(m, s);
+		m->compact_state = SVT_COMPACT_INELIGIBLE;
+		return SVTGPU_OK;
+	}
+	SVT_CUDA(e);
+	SVT_CUDA(cudaMemsetAsync(m->d_vals8 + m->nnz, 0, SVT_COMPACT_PAD, s));
+	if (m->d_offs16 != NULL)
+		SVT_CUDA(cudaMemsetAsync(m->d_offs16 + m->nnz, 0,
+					 2 * SVT_COMPACT_PAD, s));
+	const int vec = (((uintptr_t) m->d_vals) & 15) == 0 &&
+			(m->d_offs16 == NULL || (((uintptr_t) m->d_offs) & 15) == 0);
+	narrow_compact<<<(unsigned) (svtgpu_sm_count() * 8), 256, 0, s>>>(
+		m->d_offs, (const int32_t *) m->d_vals, m->d_offs16, m->d_vals8,
+		m->nnz, vec);
+	SVT_CUDA(cudaGetLastError());
+	svtgpu_count_launch(1);
+	/* later calls may come on other streams */
+	SVT_CUDA(cudaStreamSynchronize(s));
+	m->compact_state = SVT_COMPACT_BUILT;
+	return SVTGPU_OK;
+}
+
+extern "C" int svtgpu_matrix_compact_bytes(const svtgpu_matrix *m,
+					   int64_t *bytes)
+{
+	SVT_ARG(m != NULL && bytes != NULL,
+		"svtgpu_matrix_compact_bytes: NULL argument");
+	const int64_t n = m->nnz + SVT_COMPACT_PAD;
+	*bytes = (m->d_vals8 != NULL ? n : 0) + (m->d_offs16 != NULL ? 2 * n : 0);
 	return SVTGPU_OK;
 }
 

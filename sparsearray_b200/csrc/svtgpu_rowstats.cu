@@ -740,6 +740,14 @@ __device__ __forceinline__ int4 ldg_stream_v4(const int4 *p)
 	return r;
 }
 
+__device__ __forceinline__ uint2 ldg_stream_v2(const uint2 *p)
+{
+	uint2 r;
+	asm volatile("ld.global.nc.L1::no_allocate.v2.u32 {%0, %1}, [%2];"
+		     : "=r"(r.x), "=r"(r.y) : "l"(p));
+	return r;
+}
+
 /* PACKED row min / max (non-negative integers < 65535): coverage count in
  * the high, running extreme in the low 16 bits of one accumulator.  A minimum
  * is kept as the maximum of the complemented values (x ^ 0xFFFF), so both
@@ -1494,6 +1502,8 @@ int ensure_split(svtgpu_matrix *m, const TileConfig &c, cudaStream_t s,
 struct RowHistParams {
 	const int32_t *offs;
 	const int32_t *vals;       /* NULL: lacunar */
+	const uint16_t *offs16;    /* compact copy (row_hist<MODE, true>) */
+	const int8_t *vals8;
 	const int64_t *leaf_ptr;
 	int64_t nleaf, nnz, nrow;
 	int nchunks;
@@ -1525,7 +1535,7 @@ __device__ __forceinline__ void hist_red_max(uint32_t saddr, uint32_t v)
    and sum(x^2) in the high 16 bits of one cell -- piece_leaves is then what
    cannot add 2^15 to a half, and the cells are only flushed when a guard bit
    (2^15 of a half) shows, as in row_strips. */
-template <int MODE>
+template <int MODE, bool NARROW>
 __global__ void __launch_bounds__(HIST_THREADS, 1)
 row_hist(RowHistParams P)
 {
@@ -1689,6 +1699,76 @@ row_hist(RowHistParams P)
 		}
 	}
 	};
+	/* NARROW (HIST_SUM32 / HIST_MOMENTS only): the same entries from the
+	   compact copy (svtgpu_internal.h), 3 bytes each instead of 8 */
+	auto add8 = [&](const uint32_t o, const int x) {
+		if (x == SVT_COMPACT_NA_I8) {
+			atomicAdd(&P.state[SVT_ROW_SLOT_NA * P.nrow + o], 1.0);
+		} else if (MODE == HIST_MOMENTS) {
+			const unsigned int v = (unsigned int) x;
+			hist_red(cell_s + (o << 2), v * ((v << 16) + 1u));
+		} else {
+			hist_red(cell_s + (o << 2), (unsigned int) x);
+		}
+	};
+	auto stream8 = [&](const int64_t start, const int64_t end) {
+	/* single entries up to a multiple of 8, then batches in which every
+	   thread takes K groups of 8 entries (one 16-byte load of offsets and
+	   one 8-byte load of values each), double-buffered as above */
+	constexpr int K = 2;
+	int64_t head = (8 - (start & 7)) & 7;
+	if (head > end - start)
+		head = end - start;
+	if ((int64_t) threadIdx.x < head)
+		add8(P.offs16[start + threadIdx.x], P.vals8[start + threadIdx.x]);
+	const int64_t vstart = start + head;
+	const int64_t nfull = (end - vstart) / ((int64_t) HIST_THREADS * 8 * K);
+	const int4 *po = (const int4 *) (P.offs16 + vstart) + threadIdx.x;
+	const uint2 *pv = (const uint2 *) (P.vals8 + vstart) + threadIdx.x;
+	int4 o_nx[K];
+	uint2 v_nx[K];
+	auto request = [&]() {
+#pragma unroll
+		for (int k = 0; k < K; k++) {
+			o_nx[k] = ldg_stream_v4(po + k * HIST_THREADS);
+			v_nx[k] = ldg_stream_v2(pv + k * HIST_THREADS);
+		}
+		po += K * HIST_THREADS;
+		pv += K * HIST_THREADS;
+	};
+	if (nfull > 0)
+		request();
+	for (int64_t b = 0; b < nfull; b++) {
+		int4 o[K];
+		uint2 v[K];
+#pragma unroll
+		for (int k = 0; k < K; k++) {
+			o[k] = o_nx[k];
+			v[k] = v_nx[k];
+		}
+		if (b + 1 < nfull)
+			request();
+#pragma unroll
+		for (int k = 0; k < K; k++) {
+			const uint32_t ow[4] = { (uint32_t) o[k].x, (uint32_t) o[k].y,
+						 (uint32_t) o[k].z, (uint32_t) o[k].w };
+			const uint32_t vw[2] = { v[k].x, v[k].y };
+#pragma unroll
+			for (int j = 0; j < 8; j++)
+				add8((ow[j >> 1] >> ((j & 1) * 16)) & 0xFFFFu,
+				     (int) (int8_t) (vw[j >> 2] >> ((j & 3) * 8)));
+		}
+	}
+	for (int64_t e = vstart + nfull * HIST_THREADS * 8 * K + threadIdx.x;
+	     e < end; e += HIST_THREADS)
+		add8(P.offs16[e], P.vals8[e]);
+	};
+	auto feed = [&](const int64_t start, const int64_t end) {
+		if (NARROW)
+			stream8(start, end);
+		else
+			stream(start, end);
+	};
 	/* after a piece: MOMENTS keeps accumulating on chip while no guard bit
 	   shows; everything else (and the last piece) goes to the row state */
 	auto checkpoint = [&](const bool last) {
@@ -1786,8 +1866,8 @@ row_hist(RowHistParams P)
 			}
 			used += L;
 			const int64_t start = t * P.tile;
-			stream(start, start + P.tile < P.nnz ? start + P.tile
-							     : P.nnz);
+			feed(start, start + P.tile < P.nnz ? start + P.tile
+							   : P.nnz);
 			t = tn;
 			la = na;
 			lb = nb;
@@ -1825,7 +1905,7 @@ row_hist(RowHistParams P)
 		     p0 += P.piece_leaves) {
 			const int64_t p1 = p0 + P.piece_leaves < bounds[1]
 					   ? p0 + P.piece_leaves : bounds[1];
-			stream(P.leaf_ptr[p0], P.leaf_ptr[p1]);
+			feed(P.leaf_ptr[p0], P.leaf_ptr[p1]);
 			checkpoint(p1 == bounds[1]);
 		}
 	}
@@ -1870,6 +1950,13 @@ int launch_row_hist(svtgpu_matrix *m, int mode, int64_t max_abs,
 	P.nleaf = m->nleaf;
 	P.nnz = m->nnz;
 	P.nrow = m->nrow;
+	bool narrow = false;
+	if (mode == HIST_SUM32 || mode == HIST_MOMENTS) {
+		SVT_CHECK(svt_ensure_compact(m, s));
+		narrow = m->d_offs16 != NULL && m->d_vals8 != NULL;
+		P.offs16 = m->d_offs16;
+		P.vals8 = m->d_vals8;
+	}
 	const int sms = svtgpu_sm_count();
 	P.nchunks = (int64_t) sms * 2 < m->nleaf ? sms * 2
 						 : (m->nleaf > 0 ? (int) m->nleaf : 1);
@@ -1931,15 +2018,17 @@ int launch_row_hist(svtgpu_matrix *m, int mode, int64_t max_abs,
 			grid = sms;
 		}
 	}
-#define HIST_LAUNCH(MODE) do { \
-		SVT_CUDA(cudaFuncSetAttribute(row_hist<MODE>, \
+#define HIST_LAUNCH(MODE, NARROW) do { \
+		SVT_CUDA(cudaFuncSetAttribute(row_hist<MODE, NARROW>, \
 			cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem)); \
-		row_hist<MODE><<<grid, HIST_THREADS, smem, s>>>(P); \
+		row_hist<MODE, NARROW><<<grid, HIST_THREADS, smem, s>>>(P); \
 	} while (0)
-	if (mode == HIST_COUNT16)      HIST_LAUNCH(HIST_COUNT16);
-	else if (mode == HIST_MOMENTS) HIST_LAUNCH(HIST_MOMENTS);
-	else if (mode == HIST_MAX32)   HIST_LAUNCH(HIST_MAX32);
-	else                           HIST_LAUNCH(HIST_SUM32);
+	if (mode == HIST_COUNT16)      HIST_LAUNCH(HIST_COUNT16, false);
+	else if (mode == HIST_MOMENTS && narrow) HIST_LAUNCH(HIST_MOMENTS, true);
+	else if (mode == HIST_MOMENTS) HIST_LAUNCH(HIST_MOMENTS, false);
+	else if (mode == HIST_MAX32)   HIST_LAUNCH(HIST_MAX32, false);
+	else if (narrow)               HIST_LAUNCH(HIST_SUM32, true);
+	else                           HIST_LAUNCH(HIST_SUM32, false);
 #undef HIST_LAUNCH
 	SVT_CUDA(cudaGetLastError());
 	svtgpu_count_launch(1);

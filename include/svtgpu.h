@@ -337,7 +337,8 @@ int svtgpu_matmul_dev(svtgpu_matrix *m, const void *d_d_rowmajor, int d_type,
 		      int64_t K, double *d_ans_rowmajor, void *stream);
 
 /* ---- element-wise operations that keep the implicit zeros at zero ----
- * Arith `x * v`, `v * x`, `x / v` and the Math functions below, with base R's
+ * Arith `x * v`, `v * x`, `x / v`, the Math functions and the comparisons
+ * and is.* predicates below, with base R's
  * dense semantics (result types, NA / NaN, integer overflow: the rules live
  * in csrc/svt_semantics.h).  *out is a NEW matrix (owned by the caller, free
  * it with svtgpu_matrix_free()) with x's geometry; computed values equal to 0
@@ -349,11 +350,19 @@ int svtgpu_matmul_dev(svtgpu_matrix *m, const void *d_d_rowmajor, int d_type,
  *   margin:  0 = scalar (operand_len 1), 1 = operand[row] (operand_len =
  *            nrow), 2 = operand[leaf] (operand_len = nleaf: a column shard
  *            passes its own slice of the per-column vector);
- *   operand_on_left: `v * x` / `v / x` (the latter is refused).
+ *   operand_on_left: `v * x` / `v / x` (the latter is refused); for the
+ *            comparisons `v op x`, served as the mirrored `x op' v`.
  * An operation that would turn the implicit zeros into something else
  * (`x * Inf`, `x * NA`, `x / 0`, `v / x`, other opcodes) fails with
  * SVTGPU_ERR_ARG and R's wording before any device work.
- * *warn: SVTGPU_EW_WARN_* bits. */
+ * Comparisons (SVTGPU_EW_GT ... NE) and the is.* predicates
+ * (SVTGPU_EW_IS_*) give a logical result (val_type SVTGPU_LGL): an entry is
+ * stored where the value is TRUE or NA, and FALSE is dropped.  They are
+ * admitted only when `0 op v` is FALSE for every operand element (NA / NaN
+ * operands are refused).  A result with no NA has no value array (flags
+ * without SVTGPU_HAS_VALS: every leaf lacunar); one with an NA stores 1 and
+ * NA_integer_.  The is.* predicates take no operand and never hold NA.
+ * *warn: SVTGPU_EW_WARN_* bits (never set by comparisons). */
 #define SVTGPU_EW_MUL       1
 #define SVTGPU_EW_DIV       2
 #define SVTGPU_EW_ABS      11
@@ -364,6 +373,15 @@ int svtgpu_matmul_dev(svtgpu_matrix *m, const void *d_d_rowmajor, int d_type,
 #define SVTGPU_EW_TRUNC    16
 #define SVTGPU_EW_LOG1P    17
 #define SVTGPU_EW_EXPM1    18
+#define SVTGPU_EW_GT       21  /* x >  v */
+#define SVTGPU_EW_GE       22  /* x >= v */
+#define SVTGPU_EW_LT       23  /* x <  v */
+#define SVTGPU_EW_LE       24  /* x <= v */
+#define SVTGPU_EW_EQ       25  /* x == v */
+#define SVTGPU_EW_NE       26  /* x != v */
+#define SVTGPU_EW_IS_NA        31  /* is.na(x): NA or NaN */
+#define SVTGPU_EW_IS_NAN       32  /* is.nan(x): NaN that is not NA */
+#define SVTGPU_EW_IS_INFINITE  33  /* is.infinite(x) */
 #define SVTGPU_EW_WARN_INT_OVERFLOW  1  /* "NAs produced by integer overflow" */
 #define SVTGPU_EW_WARN_NAN           2  /* "NaNs produced" */
 int svtgpu_ewise(svtgpu_matrix *x, int op, const void *operand,

@@ -107,7 +107,10 @@ SIGNATURES = {
 
 # element-wise opcodes (SVTGPU_EW_*) and warning bits
 EW_OPCODES = {"*": 1, "/": 2, "abs": 11, "sign": 12, "sqrt": 13, "floor": 14,
-              "ceiling": 15, "trunc": 16, "log1p": 17, "expm1": 18}
+              "ceiling": 15, "trunc": 16, "log1p": 17, "expm1": 18,
+              ">": 21, ">=": 22, "<": 23, "<=": 24, "==": 25, "!=": 26,
+              "is.na": 31, "is.nan": 32, "is.infinite": 33}
+EW_COMPARE = (">", ">=", "<", "<=", "==", "!=")
 EW_WARN_INT_OVERFLOW, EW_WARN_NAN = 1, 2
 EW_WARNINGS = ((EW_WARN_INT_OVERFLOW, "NAs produced by integer overflow"),
                (EW_WARN_NAN, "NaNs produced"))

@@ -611,6 +611,18 @@ SVT_HD double svt_dot_finalize(int is_double, double s, int leaf_flag,
 
 /* bits OR-ed by the value rules (the first two are svtgpu_ewise's *warn) */
 #define SVT_EW_DROPPED      4  /* a computed value compares equal to 0 */
+#define SVT_EW_NA_KEPT      8  /* a comparison kept an NA entry */
+
+/* what svt_ew_cmp() makes of one stored value */
+#define SVT_CMP_DROP        0  /* FALSE: the entry leaves the result */
+#define SVT_CMP_TRUE        1
+#define SVT_CMP_NA          2
+
+/* what kind of name the caller was given (svt_ew_refusal_message()) */
+#define SVT_EW_KIND_ARITH   0
+#define SVT_EW_KIND_MATH    1
+#define SVT_EW_KIND_COMPARE 2
+#define SVT_EW_KIND_IS      3
 
 SVT_HD int svt_ew_is_arith(int op)
 {
@@ -620,6 +632,35 @@ SVT_HD int svt_ew_is_arith(int op)
 SVT_HD int svt_ew_is_math(int op)
 {
 	return op >= SVTGPU_EW_ABS && op <= SVTGPU_EW_EXPM1;
+}
+
+SVT_HD int svt_ew_is_compare(int op)
+{
+	return op >= SVTGPU_EW_GT && op <= SVTGPU_EW_NE;
+}
+
+/* is.na / is.nan / is.infinite */
+SVT_HD int svt_ew_is_pred(int op)
+{
+	return op >= SVTGPU_EW_IS_NA && op <= SVTGPU_EW_IS_INFINITE;
+}
+
+/* operations that take no operand */
+SVT_HD int svt_ew_is_unary(int op)
+{
+	return svt_ew_is_math(op) || svt_ew_is_pred(op);
+}
+
+/* `v op x` is `x op' v`: the order comparisons swap, == and != stay */
+SVT_HD int svt_ew_mirror(int op)
+{
+	switch (op) {
+	    case SVTGPU_EW_GT: return SVTGPU_EW_LT;
+	    case SVTGPU_EW_GE: return SVTGPU_EW_LE;
+	    case SVTGPU_EW_LT: return SVTGPU_EW_GT;
+	    case SVTGPU_EW_LE: return SVTGPU_EW_GE;
+	}
+	return op;
 }
 
 SVT_HD int svt_ew_streq(const char *a, const char *b)
@@ -653,6 +694,15 @@ SVT_HD const char *svt_ew_opname(int op)
 	    case SVTGPU_EW_TRUNC:   return "trunc";
 	    case SVTGPU_EW_LOG1P:   return "log1p";
 	    case SVTGPU_EW_EXPM1:   return "expm1";
+	    case SVTGPU_EW_GT:      return ">";
+	    case SVTGPU_EW_GE:      return ">=";
+	    case SVTGPU_EW_LT:      return "<";
+	    case SVTGPU_EW_LE:      return "<=";
+	    case SVTGPU_EW_EQ:      return "==";
+	    case SVTGPU_EW_NE:      return "!=";
+	    case SVTGPU_EW_IS_NA:       return "is.na";
+	    case SVTGPU_EW_IS_NAN:      return "is.nan";
+	    case SVTGPU_EW_IS_INFINITE: return "is.infinite";
 	}
 	return "?";
 }
@@ -660,6 +710,25 @@ SVT_HD const char *svt_ew_opname(int op)
 SVT_HD int svt_ew_math_opcode(const char *name)
 {
 	for (int op = SVTGPU_EW_ABS; op <= SVTGPU_EW_EXPM1; op++)
+		if (svt_ew_streq(name, svt_ew_opname(op)))
+			return op;
+	return 0;
+}
+
+/* R's Compare group (">", ">=", "<", "<=", "==", "!=") -> opcode; else 0 */
+SVT_HD int svt_ew_compare_opcode(const char *name)
+{
+	for (int op = SVTGPU_EW_GT; op <= SVTGPU_EW_NE; op++)
+		if (svt_ew_streq(name, svt_ew_opname(op)))
+			return op;
+	return 0;
+}
+
+/* "is.na", "is.nan", "is.infinite" -> opcode; any other name (is.finite
+   would make the zeros TRUE) -> 0 */
+SVT_HD int svt_ew_is_opcode(const char *name)
+{
+	for (int op = SVTGPU_EW_IS_NA; op <= SVTGPU_EW_IS_INFINITE; op++)
 		if (svt_ew_streq(name, svt_ew_opname(op)))
 			return op;
 	return 0;
@@ -675,6 +744,8 @@ SVT_HD int svt_ew_type_ok(int t)
  * logical input (do_abs()). */
 SVT_HD int svt_ew_result_type(int op, int x_type, int v_type)
 {
+	if (svt_ew_is_compare(op) || svt_ew_is_pred(op))
+		return SVTGPU_LGL;
 	if (op == SVTGPU_EW_MUL)
 		return (x_type != SVTGPU_DOUBLE && v_type != SVTGPU_DOUBLE)
 			? SVTGPU_INT : SVTGPU_DOUBLE;
@@ -683,10 +754,47 @@ SVT_HD int svt_ew_result_type(int op, int x_type, int v_type)
 	return SVTGPU_DOUBLE;
 }
 
+/* Comparison or is.* predicate of one stored value (base R's relop.c and
+ * do_isna() / do_isnan() / do_isinfinite()): SVT_CMP_TRUE, SVT_CMP_NA or
+ * SVT_CMP_DROP (FALSE).  x: the value as a double (an int32 converts
+ * exactly, so int op int compares as R does); x_na: the value is NA
+ * (NA_integer_ or R_IsNA()).  v: the operand element as a double (never NA
+ * or NaN once admitted), ignored by the predicates.  An NA or NaN value
+ * compares to NA; is.na() is TRUE for both, is.nan() for a NaN that is not
+ * NA. */
+SVT_HD int svt_ew_cmp(int op, double x, int x_na, double v)
+{
+	switch (op) {
+	    case SVTGPU_EW_IS_NA:
+		return (x_na || svt_isnan(x)) ? SVT_CMP_TRUE : SVT_CMP_DROP;
+	    case SVTGPU_EW_IS_NAN:
+		return (!x_na && svt_isnan(x)) ? SVT_CMP_TRUE : SVT_CMP_DROP;
+	    case SVTGPU_EW_IS_INFINITE:
+		return (!x_na && (x == svt_posinf() || x == svt_neginf()))
+			? SVT_CMP_TRUE : SVT_CMP_DROP;
+	}
+	if (x_na || svt_isnan(x) || svt_isnan(v))
+		return SVT_CMP_NA;
+	bool r;
+	switch (op) {
+	    case SVTGPU_EW_GT: r = x >  v; break;
+	    case SVTGPU_EW_GE: r = x >= v; break;
+	    case SVTGPU_EW_LT: r = x <  v; break;
+	    case SVTGPU_EW_LE: r = x <= v; break;
+	    case SVTGPU_EW_EQ: r = x == v; break;
+	    case SVTGPU_EW_NE: r = x != v; break;
+	    default:           return SVT_CMP_NA;
+	}
+	return r ? SVT_CMP_TRUE : SVT_CMP_DROP;
+}
+
 /* Would f(0) stay 0 for every element of the operand?  Arith ops only.
  *   margin 0: v is a scalar; 1: v[i] for row i (R's recycling of `x op v`
  *   with length(v) == nrow, any number of dimensions); 2: v[j] for column j
  *   (`sweep(x, 2, v, op)`, 2-D only; nleaf columns).
+ * Comparisons (`v op x` mirrored first) need `0 op v` FALSE for every
+ * element: v >= 0 for ">", v > 0 for ">=", v <= 0 for "<", v < 0 for "<=",
+ * v != 0 for "==", v == 0 for "!="; NA and NaN never (0 op NA is NA).
  * Returns SVT_EW_OK or a refusal code; *bad receives the offending element
  * for SVT_EW_BAD_VALUE. */
 SVT_HD int svt_ew_check(int op, int x_type, int v_type, int64_t v_len,
@@ -696,10 +804,13 @@ SVT_HD int svt_ew_check(int op, int x_type, int v_type, int64_t v_len,
 	*bad = -1;
 	if (!svt_ew_type_ok(x_type))
 		return SVT_EW_BAD_X_TYPE;
-	if (svt_ew_is_math(op))
+	if (svt_ew_is_unary(op))
 		return SVT_EW_OK;
-	if (!svt_ew_is_arith(op))
+	const int cmp = svt_ew_is_compare(op);
+	if (!svt_ew_is_arith(op) && !cmp)
 		return SVT_EW_BAD_OPCODE;
+	if (cmp && v_on_left)
+		op = svt_ew_mirror(op);
 	if (op == SVTGPU_EW_DIV && v_on_left)
 		return SVT_EW_LEFT_DIV;
 	if (!svt_ew_type_ok(v_type))
@@ -711,7 +822,13 @@ SVT_HD int svt_ew_check(int op, int x_type, int v_type, int64_t v_len,
 		return SVT_EW_BAD_LENGTH;
 	for (int64_t i = 0; i < v_len; i++) {
 		int ok;
-		if (v_type == SVTGPU_DOUBLE) {
+		if (cmp) {
+			const double d = v_type == SVTGPU_DOUBLE
+				? ((const double *) v)[i]
+				: (((const int32_t *) v)[i] == SVT_NA_INT ? svt_nan()
+					: (double) ((const int32_t *) v)[i]);
+			ok = svt_ew_cmp(op, 0.0, 0, d) == SVT_CMP_DROP;
+		} else if (v_type == SVTGPU_DOUBLE) {
 			const double d = ((const double *) v)[i];
 			/* 0 * Inf is NaN, 0 * NA is NA; 0 / 0 is NaN, 0 / NA
 			   is NA; 0 / Inf is 0 */
@@ -729,30 +846,51 @@ SVT_HD int svt_ew_check(int op, int x_type, int v_type, int64_t v_len,
 	return SVT_EW_OK;
 }
 
-static inline const char *svt_ew_value_name(int v_type, const void *v,
-					    int64_t i)
+/* operand element i as R prints it; `lgl_words`: logical as TRUE / FALSE */
+static inline void svt_ew_value_name(int v_type, const void *v, int64_t i,
+				     int lgl_words, char *buf, size_t len)
 {
-	if (v_type != SVTGPU_DOUBLE)
-		return ((const int32_t *) v)[i] == SVT_NA_INT ? "NA" : "0";
+	if (v_type != SVTGPU_DOUBLE) {
+		const int32_t k = ((const int32_t *) v)[i];
+		if (k == SVT_NA_INT)
+			snprintf(buf, len, "NA");
+		else if (v_type == SVTGPU_LGL && lgl_words)
+			snprintf(buf, len, "%s", k ? "TRUE" : "FALSE");
+		else
+			snprintf(buf, len, "%d", (int) k);
+		return;
+	}
 	const double d = ((const double *) v)[i];
-	if (svt_is_na_real(d)) return "NA";
-	if (svt_isnan(d)) return "NaN";
-	if (d == svt_posinf()) return "Inf";
-	if (d == svt_neginf()) return "-Inf";
-	return "0";
+	if (svt_is_na_real(d))       snprintf(buf, len, "NA");
+	else if (svt_isnan(d))       snprintf(buf, len, "NaN");
+	else if (d == svt_posinf())  snprintf(buf, len, "Inf");
+	else if (d == svt_neginf())  snprintf(buf, len, "-Inf");
+	else                         snprintf(buf, len, "%.15g", d);
 }
 
 /* The R error message of a refusal (host only).  `opname` is the name the
- * caller was given (it may be an operator svt_ew_check() does not know). */
+ * caller was given (it may be an operator svt_ew_check() does not know);
+ * `kind` (SVT_EW_KIND_*) the group it was given as. */
 static inline void svt_ew_refusal_message(int code, const char *opname,
-					  int is_math, int op, int v_type, const void *v,
+					  int kind, int op, int v_type, const void *v,
 					  int64_t v_len, int margin,
 					  int64_t nrow, int64_t nleaf,
 					  int64_t bad, char *buf, size_t len)
 {
+	char vname[40];
 	switch (code) {
 	    case SVT_EW_BAD_OPCODE:
-		if (is_math)
+		if (kind == SVT_EW_KIND_COMPARE)
+			snprintf(buf, len, "Compare operator \"%s\" is not "
+				 "supported on a SparseArray on the GPU path "
+				 "(supported: \">\", \">=\", \"<\", \"<=\", "
+				 "\"==\", \"!=\")", opname);
+		else if (kind == SVT_EW_KIND_IS)
+			snprintf(buf, len, "\"%s\" is not supported on a "
+				 "SparseArray on the GPU path: it would turn the "
+				 "implicit zeros into TRUE or is not a predicate "
+				 "(supported: is.na, is.nan, is.infinite)", opname);
+		else if (kind == SVT_EW_KIND_MATH)
 			snprintf(buf, len, "Math function \"%s\" is not supported "
 				 "on a SparseArray on the GPU path: it does not "
 				 "map zero to zero (supported: abs, sign, sqrt, "
@@ -794,14 +932,19 @@ static inline void svt_ew_refusal_message(int code, const char *opname,
 				 margin == 1 ? "nrow(x)" : "ncol(x)",
 				 (long long) (margin == 1 ? nrow : nleaf));
 		return;
-	    case SVT_EW_BAD_VALUE:
+	    case SVT_EW_BAD_VALUE: {
+		const int cmp = svt_ew_is_compare(op);
+		svt_ew_value_name(v_type, v, bad, cmp, vname, sizeof(vname));
+		const char *zeros = op == SVTGPU_EW_MUL
+			? "NaN or NA (0 * Inf, 0 * NA)" : "NaN or NA (0 / 0, 0 / NA)";
+		if (cmp)
+			zeros = (strcmp(vname, "NA") == 0 || strcmp(vname, "NaN") == 0)
+				? "NA" : "TRUE";
 		snprintf(buf, len, "operator \"%s\": element %lld of the operand "
 			 "is %s, so the implicit zeros of the result would be "
-			 "%s", opname, (long long) bad + 1,
-			 svt_ew_value_name(v_type, v, bad),
-			 op == SVTGPU_EW_MUL ? "NaN or NA (0 * Inf, 0 * NA)"
-					     : "NaN or NA (0 / 0, 0 / NA)");
+			 "%s", opname, (long long) bad + 1, vname, zeros);
 		return;
+	    }
 	}
 	snprintf(buf, len, "operator \"%s\": refused (code %d)", opname, code);
 }

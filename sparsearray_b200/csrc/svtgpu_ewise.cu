@@ -18,9 +18,14 @@
  * are OR-ed into one device word.
  *
  * Compaction, only when a value became 0: a warp per leaf counts the kept
- * entries (ballot + popc), svtgpu_exclusive_scan gives the new leaf_ptr and
- * a second warp-per-leaf pass copies the kept entries, in order, into arrays
- * of the exact size; the first pass's arrays are freed.
+ * entries, svtgpu_exclusive_scan gives the new leaf_ptr and a second
+ * warp-per-leaf pass copies the kept entries, in order, into arrays of the
+ * exact size; the first pass's arrays are freed.
+ *
+ * Comparisons (x > v, ..., x != v) and is.na / is.nan / is.infinite are the
+ * same compaction applied to x itself, a filter with a logical result: the
+ * entries where the value is TRUE or NA survive, stored as 1 / NA_integer_
+ * only when an NA survived (otherwise the result has no value array).
  */
 #include "svtgpu_internal.h"
 
@@ -187,54 +192,230 @@ ewise_map(EwParams P)
 		atomicOr(P.flags, fl);
 }
 
-/* entries of each leaf whose value is not 0 (NaN and NA are not 0) */
-template <typename TOut>
+/* ---- compaction: count -> scan -> stable copy ----
+ * What is kept is a "keep rule" K:
+ *   KeepNonzero<T>  a computed value array (Arith / Math): keep value != 0
+ *                   (NaN and NA are not 0) and copy the value;
+ *   KeepCmp<IN, M>  a comparison or is.* predicate of x's own values against
+ *                   the operand (svt_ew_cmp()): keep TRUE and NA, write 1 or
+ *                   NA_integer_ (only when the result stores values).
+ * Every rule gives, per entry, SVT_CMP_DROP / SVT_CMP_TRUE / SVT_CMP_NA:
+ *   leaf_operand(leaf)       the operand of a whole leaf (margin 0 / 2);
+ *   cls1(e, off, vl)         one entry;
+ *   load4(e, R) / cls4(R, vl, c)  four entries from 16-byte loads (e is a
+ *                            multiple of 4, so the loads are aligned);
+ *   out(e, c)                the value written for a kept entry. */
+template <typename T>
+struct KeepNonzero {
+	typedef T TOut;
+	struct Raw { T x[4]; };
+	static constexpr int BATCH = 4;     /* quads in flight per lane */
+	const T *vals;
+	__device__ __forceinline__ double leaf_operand(int64_t) const { return 0.0; }
+	__device__ __forceinline__ int cls1(int64_t e, int32_t, double) const
+	{
+		return vals[e] != (T) 0 ? SVT_CMP_TRUE : SVT_CMP_DROP;
+	}
+	__device__ __forceinline__ void load4(int64_t e, Raw &r) const
+	{
+		if (sizeof(T) == 4) {
+			const int4 q = __ldcs((const int4 *) (vals + e));
+			r.x[0] = (T) q.x; r.x[1] = (T) q.y;
+			r.x[2] = (T) q.z; r.x[3] = (T) q.w;
+		} else {
+			const double2 *p = (const double2 *) (vals + e);
+			const double2 a = __ldcs(p), b = __ldcs(p + 1);
+			r.x[0] = (T) a.x; r.x[1] = (T) a.y;
+			r.x[2] = (T) b.x; r.x[3] = (T) b.y;
+		}
+	}
+	__device__ __forceinline__ void cls4(const Raw &r, double, int c[4]) const
+	{
+		#pragma unroll
+		for (int j = 0; j < 4; j++)
+			c[j] = r.x[j] != (T) 0 ? SVT_CMP_TRUE : SVT_CMP_DROP;
+	}
+	__device__ __forceinline__ T out(int64_t e, int) const { return vals[e]; }
+	__device__ __forceinline__ int32_t off_at(int64_t) const { return 0; }
+};
+
+template <int IN, int MARGIN>
+struct KeepCmp {
+	typedef int32_t TOut;
+	struct Raw { int4 o; int4 xi; double2 xa, xb; };
+	/* offsets alone (a lacunar x) are light enough for 8; with 4, ptxas
+	   spills 8 bytes in the margin-1 form */
+	static constexpr int BATCH = IN == EW_IN_ONES ? 8 : 4;
+	const int32_t *offs;
+	const void *vals;
+	const double *v;      /* operand as doubles (margin 1: nrow, 2: nleaf) */
+	double v0;
+	int op;
+	__device__ __forceinline__ double leaf_operand(int64_t leaf) const
+	{
+		return MARGIN == 2 ? __ldg(v + leaf) : v0;
+	}
+	__device__ __forceinline__ int one(double x, int na, int32_t off,
+					   double vl) const
+	{
+		return svt_ew_cmp(op, x, na, MARGIN == 1 ? __ldg(v + off) : vl);
+	}
+	__device__ __forceinline__ int cls_int(int32_t k, int32_t off,
+					       double vl) const
+	{
+		return one((double) k, k == SVT_NA_INT, off, vl);
+	}
+	__device__ __forceinline__ int cls_dbl(double d, int32_t off,
+					       double vl) const
+	{
+		return one(d, svt_is_na_real(d), off, vl);
+	}
+	__device__ __forceinline__ int cls1(int64_t e, int32_t off,
+					    double vl) const
+	{
+		if (IN == EW_IN_INT)
+			return cls_int(((const int32_t *) vals)[e], off, vl);
+		if (IN == EW_IN_DBL)
+			return cls_dbl(((const double *) vals)[e], off, vl);
+		return one(1.0, 0, off, vl);
+	}
+	__device__ __forceinline__ void load4(int64_t e, Raw &r) const
+	{
+		r.o = MARGIN == 1 ? __ldcs((const int4 *) (offs + e))
+				  : make_int4(0, 0, 0, 0);
+		if (IN == EW_IN_INT)
+			r.xi = __ldcs((const int4 *) ((const int32_t *) vals + e));
+		if (IN == EW_IN_DBL) {
+			const double2 *p = (const double2 *)
+				((const double *) vals + e);
+			r.xa = __ldcs(p);
+			r.xb = __ldcs(p + 1);
+		}
+	}
+	__device__ __forceinline__ void cls4(const Raw &r, double vl,
+					     int c[4]) const
+	{
+		if (IN == EW_IN_INT) {
+			c[0] = cls_int(r.xi.x, r.o.x, vl);
+			c[1] = cls_int(r.xi.y, r.o.y, vl);
+			c[2] = cls_int(r.xi.z, r.o.z, vl);
+			c[3] = cls_int(r.xi.w, r.o.w, vl);
+		} else if (IN == EW_IN_DBL) {
+			c[0] = cls_dbl(r.xa.x, r.o.x, vl);
+			c[1] = cls_dbl(r.xa.y, r.o.y, vl);
+			c[2] = cls_dbl(r.xb.x, r.o.z, vl);
+			c[3] = cls_dbl(r.xb.y, r.o.w, vl);
+		} else {
+			c[0] = one(1.0, 0, r.o.x, vl);
+			c[1] = one(1.0, 0, r.o.y, vl);
+			c[2] = one(1.0, 0, r.o.z, vl);
+			c[3] = one(1.0, 0, r.o.w, vl);
+		}
+	}
+	__device__ __forceinline__ int32_t out(int64_t, int c) const
+	{
+		return c == SVT_CMP_NA ? SVT_NA_INT : 1;
+	}
+	__device__ __forceinline__ int32_t off_at(int64_t e) const
+	{
+		return MARGIN == 1 ? offs[e] : 0;
+	}
+};
+
+/* Count pass, a warp per leaf: the kept entries of every leaf; OR-s
+ * SVT_EW_DROPPED (something was dropped) and SVT_EW_NA_KEPT into *flags.
+ * The 4-aligned middle of a leaf is read as quads (16-byte loads,
+ * K::BATCH of them in flight per lane), the at most 3 + 3 entries at its
+ * ends by single lanes. */
+template <class K>
 __global__ void __launch_bounds__(256)
-ewise_count_kept(const int64_t *__restrict__ leaf_ptr,
-		 const TOut *__restrict__ vals, int64_t nleaf,
-		 int64_t *__restrict__ counts)
+ewise_count_kept(const int64_t *__restrict__ leaf_ptr, int64_t nleaf, K k,
+		 int64_t *__restrict__ counts, uint32_t *__restrict__ flags)
 {
 	const int lane = threadIdx.x & 31;
 	const int64_t warps = ((int64_t) gridDim.x * blockDim.x) >> 5;
 	const int64_t gw = ((int64_t) blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+	uint32_t fl = 0;
 	for (int64_t leaf = gw; leaf < nleaf; leaf += warps) {
 		const int64_t a = leaf_ptr[leaf], b = leaf_ptr[leaf + 1];
-		int64_t n = 0;
-		for (int64_t e0 = a; e0 < b; e0 += 32) {
-			const int64_t e = e0 + lane;
-			const bool keep = e < b && vals[e] != (TOut) 0;
-			n += __popc(__ballot_sync(0xFFFFFFFFu, keep));
+		const int64_t a4r = (a + 3) & ~(int64_t) 3;
+		const int64_t a4 = a4r < b ? a4r : b;
+		const int64_t b4r = b & ~(int64_t) 3;
+		const int64_t b4 = b4r > a4 ? b4r : a4;
+		const double vl = k.leaf_operand(leaf);
+		unsigned n = 0;
+		int c;
+		/* head [a, a4) and tail [b4, b) */
+		if (lane < 8) {
+			const int64_t e = lane < 4 ? a + lane : b4 + (lane - 4);
+			if (e < (lane < 4 ? a4 : b)) {
+				c = k.cls1(e, k.off_at(e), vl);
+				n += c != SVT_CMP_DROP;
+				fl |= c == SVT_CMP_NA ? SVT_EW_NA_KEPT
+				    : c == SVT_CMP_DROP ? SVT_EW_DROPPED : 0u;
+			}
 		}
+		const int64_t nq = (b4 - a4) >> 2;
+		#pragma unroll 1
+		for (int64_t q0 = lane; q0 < nq; q0 += 32 * K::BATCH) {
+			typename K::Raw r[K::BATCH];
+			#pragma unroll
+			for (int j = 0; j < K::BATCH; j++)
+				if (q0 + 32 * j < nq)
+					k.load4(a4 + 4 * (q0 + 32 * j), r[j]);
+			#pragma unroll
+			for (int j = 0; j < K::BATCH; j++) {
+				if (q0 + 32 * j >= nq)
+					continue;
+				int cc[4];
+				k.cls4(r[j], vl, cc);
+				#pragma unroll
+				for (int t = 0; t < 4; t++) {
+					n += cc[t] != SVT_CMP_DROP;
+					fl |= cc[t] == SVT_CMP_NA ? SVT_EW_NA_KEPT
+					    : cc[t] == SVT_CMP_DROP ? SVT_EW_DROPPED
+					    : 0u;
+				}
+			}
+		}
+		n = __reduce_add_sync(0xFFFFFFFFu, n);
 		if (lane == 0)
-			counts[leaf] = n;
+			counts[leaf] = (int64_t) n;
 	}
+	fl = __reduce_or_sync(0xFFFFFFFFu, fl);
+	if (lane == 0 && fl != 0)
+		atomicOr(flags, fl);
 }
 
-/* stable copy of the kept entries of every leaf to its new range */
-template <typename TOut>
+/* Write pass, a warp per leaf: stable copy of the kept entries of every
+ * leaf to its new range (offsets, and values when out_vals is not NULL). */
+template <class K>
 __global__ void __launch_bounds__(256)
 ewise_compact(const int64_t *__restrict__ old_ptr,
 	      const int64_t *__restrict__ new_ptr,
-	      const int32_t *__restrict__ offs, const TOut *__restrict__ vals,
-	      int32_t *__restrict__ out_offs, TOut *__restrict__ out_vals,
-	      int64_t nleaf)
+	      const int32_t *__restrict__ offs, K k,
+	      int32_t *__restrict__ out_offs,
+	      typename K::TOut *__restrict__ out_vals, int64_t nleaf)
 {
 	const int lane = threadIdx.x & 31;
 	const int64_t warps = ((int64_t) gridDim.x * blockDim.x) >> 5;
 	const int64_t gw = ((int64_t) blockIdx.x * blockDim.x + threadIdx.x) >> 5;
 	for (int64_t leaf = gw; leaf < nleaf; leaf += warps) {
 		const int64_t a = old_ptr[leaf], b = old_ptr[leaf + 1];
+		const double vl = k.leaf_operand(leaf);
 		int64_t w = new_ptr[leaf];
 		for (int64_t e0 = a; e0 < b; e0 += 32) {
 			const int64_t e = e0 + lane;
 			const bool ok = e < b;
-			const TOut x = ok ? vals[e] : (TOut) 0;
-			const bool keep = ok && x != (TOut) 0;
+			const int32_t off = ok ? offs[e] : 0;
+			const int c = ok ? k.cls1(e, off, vl) : SVT_CMP_DROP;
+			const bool keep = c != SVT_CMP_DROP;
 			const unsigned m = __ballot_sync(0xFFFFFFFFu, keep);
 			if (keep) {
 				const int64_t pos = w + __popc(m & ((1u << lane) - 1u));
-				out_offs[pos] = offs[e];
-				out_vals[pos] = x;
+				out_offs[pos] = off;
+				if (out_vals != NULL)
+					out_vals[pos] = k.out(e, c);
 			}
 			w += __popc(m);
 		}
@@ -272,7 +453,7 @@ static void launch_map(int margin, int64_t ntiles, cudaStream_t s,
 }
 
 /* the operand as the kernels read it: int32 for an integer result, else
-   double (no NA: refused before) */
+   double (no NA: refused before); comparisons pass SVTGPU_DOUBLE */
 static void *ew_host_operand(const void *operand, int operand_type,
 			     int64_t len, int out_type, size_t *bytes)
 {
@@ -373,14 +554,15 @@ static int ewise_run(svtgpu_matrix *x, int op, const void *operand,
 					 sizeof(int64_t) * (size_t) (2 * nleaf + 1),
 					 s));
 		int64_t *d_counts = W->d_counts, *d_ptr = W->d_counts + nleaf;
+		uint32_t *d_flags = (uint32_t *) W->d_aux;
+		KeepNonzero<double> kd = { (const double *) m1->d_vals };
+		KeepNonzero<int32_t> ki = { (const int32_t *) m1->d_vals };
 		if (dbl)
-			ewise_count_kept<double><<<grid, 256, 0, s>>>(
-				m1->d_leaf_ptr, (const double *) m1->d_vals, nleaf,
-				d_counts);
+			ewise_count_kept<<<grid, 256, 0, s>>>(m1->d_leaf_ptr,
+				nleaf, kd, d_counts, d_flags);
 		else
-			ewise_count_kept<int32_t><<<grid, 256, 0, s>>>(
-				m1->d_leaf_ptr, (const int32_t *) m1->d_vals,
-				nleaf, d_counts);
+			ewise_count_kept<<<grid, 256, 0, s>>>(m1->d_leaf_ptr,
+				nleaf, ki, d_counts, d_flags);
 		SVT_CUDA(cudaGetLastError());
 		svtgpu_count_launch(1);
 		SVT_CHECK(svtgpu_exclusive_scan(d_counts, nleaf, d_ptr, s));
@@ -399,15 +581,13 @@ static int ewise_run(svtgpu_matrix *x, int op, const void *operand,
 					 cudaMemcpyDeviceToDevice, s));
 		if (nnz_new > 0) {
 			if (dbl)
-				ewise_compact<double><<<grid, 256, 0, s>>>(
-					m1->d_leaf_ptr, d_ptr, m1->d_offs,
-					(const double *) m1->d_vals, m2->d_offs,
-					(double *) m2->d_vals, nleaf);
+				ewise_compact<<<grid, 256, 0, s>>>(
+					m1->d_leaf_ptr, d_ptr, m1->d_offs, kd,
+					m2->d_offs, (double *) m2->d_vals, nleaf);
 			else
-				ewise_compact<int32_t><<<grid, 256, 0, s>>>(
-					m1->d_leaf_ptr, d_ptr, m1->d_offs,
-					(const int32_t *) m1->d_vals, m2->d_offs,
-					(int32_t *) m2->d_vals, nleaf);
+				ewise_compact<<<grid, 256, 0, s>>>(
+					m1->d_leaf_ptr, d_ptr, m1->d_offs, ki,
+					m2->d_offs, (int32_t *) m2->d_vals, nleaf);
 			SVT_CUDA(cudaGetLastError());
 			svtgpu_count_launch(1);
 			launches++;
@@ -433,6 +613,182 @@ static int ewise_run(svtgpu_matrix *x, int op, const void *operand,
 	return SVTGPU_OK;
 }
 
+/* ---- comparisons and is.* predicates: a filter of x's entries ----
+ * Count pass (rule KeepCmp) -> flags; then
+ *   nothing dropped, no NA: leaf_ptr and offsets copied, no value array;
+ *   otherwise scan + write pass, values (1 / NA) only when an NA was kept.
+ * A lacunar x under a scalar operand (and is.nan / is.infinite of integer
+ * values) needs no pass at all: the predicate is a constant. */
+template <int IN, int MARGIN>
+static void cmp_launch(const svtgpu_matrix *x, int op, const double *d_v,
+		       double v0, bool write, const int64_t *d_ptr,
+		       svtgpu_matrix *m, int64_t *d_counts, uint32_t *d_flags,
+		       unsigned grid, cudaStream_t s)
+{
+	KeepCmp<IN, MARGIN> k;
+	k.offs = x->d_offs;
+	k.vals = x->d_vals;
+	k.v = d_v;
+	k.v0 = v0;
+	k.op = op;
+	if (!write)
+		ewise_count_kept<<<grid, 256, 0, s>>>(x->d_leaf_ptr, x->nleaf, k,
+						      d_counts, d_flags);
+	else
+		ewise_compact<<<grid, 256, 0, s>>>(x->d_leaf_ptr, d_ptr,
+			x->d_offs, k, m->d_offs,
+			(m->flags & SVTGPU_HAS_VALS) ? (int32_t *) m->d_vals : NULL,
+			x->nleaf);
+}
+
+template <int IN>
+static void cmp_launch_m(int margin, const svtgpu_matrix *x, int op,
+			 const double *d_v, double v0, bool write,
+			 const int64_t *d_ptr, svtgpu_matrix *m,
+			 int64_t *d_counts, uint32_t *d_flags, unsigned grid,
+			 cudaStream_t s)
+{
+	if (margin == 0)
+		cmp_launch<IN, 0>(x, op, d_v, v0, write, d_ptr, m, d_counts,
+				  d_flags, grid, s);
+	else if (margin == 1)
+		cmp_launch<IN, 1>(x, op, d_v, v0, write, d_ptr, m, d_counts,
+				  d_flags, grid, s);
+	else
+		cmp_launch<IN, 2>(x, op, d_v, v0, write, d_ptr, m, d_counts,
+				  d_flags, grid, s);
+}
+
+/* a logical result of x's geometry: leaf_ptr and offsets copied from x
+   (everything kept), or nnz = 0 (nothing kept) */
+static int cmp_result_copy(svtgpu_matrix *x, bool keep_all, EwWork *W,
+			   cudaStream_t s)
+{
+	const int64_t nnz = keep_all ? x->nnz : 0;
+	SVT_CHECK(svtgpu_matrix_create(&W->m2, x->nrow, x->nleaf, nnz,
+				       SVTGPU_LGL, nnz > 0 ? SVTGPU_HAS_OFFS : 0));
+	svtgpu_matrix *m = W->m2;
+	SVT_CUDA(cudaStreamSynchronize(m->up_stream));
+	const size_t lp_bytes = sizeof(int64_t) * (size_t) (x->nleaf + 1);
+	if (keep_all)
+		SVT_CUDA(cudaMemcpyAsync(m->d_leaf_ptr, x->d_leaf_ptr, lp_bytes,
+					 cudaMemcpyDeviceToDevice, s));
+	else
+		SVT_CUDA(cudaMemsetAsync(m->d_leaf_ptr, 0, lp_bytes, s));
+	if (nnz > 0)
+		SVT_CUDA(cudaMemcpyAsync(m->d_offs, x->d_offs,
+					 sizeof(int32_t) * (size_t) nnz,
+					 cudaMemcpyDeviceToDevice, s));
+	return SVTGPU_OK;
+}
+
+static int compare_run(svtgpu_matrix *x, int op, const void *operand,
+		       int operand_type, int64_t operand_len, int margin,
+		       EwWork *W, svtgpu_matrix **out)
+{
+	cudaStream_t s = 0;
+	const int64_t nnz = x->nnz, nleaf = x->nleaf;
+	const int in = ((x->flags & SVTGPU_HAS_VALS) && x->d_vals != NULL)
+		? (svt_is_double(x->val_type) ? EW_IN_DBL : EW_IN_INT)
+		: EW_IN_ONES;
+	const int64_t vlen = svt_ew_is_pred(op) ? 0 : operand_len;
+	size_t op_bytes = 0;
+	W->h_op = ew_host_operand(operand, operand_type, vlen, SVTGPU_DOUBLE,
+				  &op_bytes);
+	if (W->h_op == NULL) {
+		svtgpu_set_error("svtgpu_ewise: out of host memory");
+		return SVTGPU_ERR_NOMEM;
+	}
+	const double v0 = ((const double *) W->h_op)[0];
+	/* a constant predicate: every entry of x gives the same answer */
+	int konst = -1;
+	if (in == EW_IN_ONES && (margin == 0 || svt_ew_is_pred(op)))
+		konst = svt_ew_cmp(op, 1.0, 0, v0);
+	else if (in == EW_IN_INT && (op == SVTGPU_EW_IS_NAN ||
+				     op == SVTGPU_EW_IS_INFINITE))
+		konst = SVT_CMP_DROP;
+	if (nnz == 0)
+		konst = SVT_CMP_TRUE;
+	SvtTimer tm;
+	SVT_CHECK(svt_timer_begin(&tm, s));
+	int launches = 0;
+	if (konst >= 0) {
+		SVT_CHECK(cmp_result_copy(x, konst != SVT_CMP_DROP, W, s));
+	} else {
+		const unsigned grid = (unsigned) (svtgpu_sm_count() * 8);
+		SVT_CUDA(svt_malloc_async(&W->d_aux, 16 + op_bytes, s));
+		uint32_t *d_flags = (uint32_t *) W->d_aux;
+		double *d_v = (double *) ((char *) W->d_aux + 16);
+		SVT_CUDA(cudaMemsetAsync(d_flags, 0, 16, s));
+		SVT_CUDA(cudaMemcpyAsync(d_v, W->h_op, op_bytes,
+					 cudaMemcpyHostToDevice, s));
+		SVT_CUDA(svt_malloc_async((void **) &W->d_counts,
+					 sizeof(int64_t) * (size_t) (2 * nleaf + 1),
+					 s));
+		int64_t *d_counts = W->d_counts, *d_ptr = W->d_counts + nleaf;
+		if (in == EW_IN_DBL)
+			cmp_launch_m<EW_IN_DBL>(margin, x, op, d_v, v0, false, NULL,
+						NULL, d_counts, d_flags, grid, s);
+		else if (in == EW_IN_INT)
+			cmp_launch_m<EW_IN_INT>(margin, x, op, d_v, v0, false, NULL,
+						NULL, d_counts, d_flags, grid, s);
+		else
+			cmp_launch_m<EW_IN_ONES>(margin, x, op, d_v, v0, false,
+						 NULL, NULL, d_counts, d_flags,
+						 grid, s);
+		SVT_CUDA(cudaGetLastError());
+		svtgpu_count_launch(1);
+		launches++;
+		uint32_t flags = 0;
+		SVT_CUDA(cudaMemcpyAsync(&flags, d_flags, sizeof(flags),
+					 cudaMemcpyDeviceToHost, s));
+		SVT_CUDA(cudaStreamSynchronize(s));
+		if (!(flags & (SVT_EW_DROPPED | SVT_EW_NA_KEPT))) {
+			SVT_CHECK(cmp_result_copy(x, true, W, s));
+		} else {
+			SVT_CHECK(svtgpu_exclusive_scan(d_counts, nleaf, d_ptr, s));
+			launches += 2;
+			int64_t nnz_new = 0;
+			SVT_CUDA(cudaMemcpyAsync(&nnz_new, d_ptr + nleaf,
+						 sizeof(int64_t),
+						 cudaMemcpyDeviceToHost, s));
+			SVT_CUDA(cudaStreamSynchronize(s));
+			const int fl = nnz_new == 0 ? 0 : SVTGPU_HAS_OFFS |
+				((flags & SVT_EW_NA_KEPT) ? SVTGPU_HAS_VALS : 0);
+			SVT_CHECK(svtgpu_matrix_create(&W->m2, x->nrow, nleaf,
+						       nnz_new, SVTGPU_LGL, fl));
+			svtgpu_matrix *m = W->m2;
+			SVT_CUDA(cudaStreamSynchronize(m->up_stream));
+			SVT_CUDA(cudaMemcpyAsync(m->d_leaf_ptr, d_ptr,
+						 sizeof(int64_t) * (size_t) (nleaf + 1),
+						 cudaMemcpyDeviceToDevice, s));
+			if (nnz_new > 0) {
+				if (in == EW_IN_DBL)
+					cmp_launch_m<EW_IN_DBL>(margin, x, op, d_v,
+						v0, true, d_ptr, m, NULL, NULL, grid, s);
+				else if (in == EW_IN_INT)
+					cmp_launch_m<EW_IN_INT>(margin, x, op, d_v,
+						v0, true, d_ptr, m, NULL, NULL, grid, s);
+				else
+					cmp_launch_m<EW_IN_ONES>(margin, x, op, d_v,
+						v0, true, d_ptr, m, NULL, NULL, grid, s);
+				SVT_CUDA(cudaGetLastError());
+				svtgpu_count_launch(1);
+				launches++;
+			}
+		}
+	}
+	double ms = 0.0;
+	SVT_CHECK(svt_timer_end(&tm, &ms));
+	svtgpu_matrix *res = W->m2;
+	W->m2 = NULL;
+	res->leaf_base = x->leaf_base;
+	res->tm.kernel_ms = ms;
+	res->tm.launches = launches;
+	*out = res;
+	return SVTGPU_OK;
+}
+
 extern "C" int svtgpu_ewise(svtgpu_matrix *x, int op, const void *operand,
 			    int operand_type, int64_t operand_len, int margin,
 			    int operand_on_left, svtgpu_matrix **out, int *warn)
@@ -442,7 +798,7 @@ extern "C" int svtgpu_ewise(svtgpu_matrix *x, int op, const void *operand,
 	if (warn != NULL)
 		*warn = 0;
 	const int is_math = svt_ew_is_math(op);
-	SVT_ARG(is_math || operand != NULL || operand_len == 0,
+	SVT_ARG(svt_ew_is_unary(op) || operand != NULL || operand_len == 0,
 		"svtgpu_ewise: NULL operand");
 	int64_t bad = -1;
 	const int code = svt_ew_check(op, x->val_type, operand_type,
@@ -450,7 +806,10 @@ extern "C" int svtgpu_ewise(svtgpu_matrix *x, int op, const void *operand,
 				      x->nrow, x->nleaf, operand, &bad);
 	if (code != SVT_EW_OK) {
 		char msg[512];
-		svt_ew_refusal_message(code, svt_ew_opname(op), is_math, op,
+		const int kind = is_math ? SVT_EW_KIND_MATH
+			: svt_ew_is_compare(op) ? SVT_EW_KIND_COMPARE
+			: svt_ew_is_pred(op) ? SVT_EW_KIND_IS : SVT_EW_KIND_ARITH;
+		svt_ew_refusal_message(code, svt_ew_opname(op), kind, op,
 				       operand_type, operand, operand_len,
 				       margin, x->nrow, x->nleaf, bad, msg,
 				       sizeof(msg));
@@ -467,8 +826,11 @@ extern "C" int svtgpu_ewise(svtgpu_matrix *x, int op, const void *operand,
 	const int out_type = svt_ew_result_type(op, x->val_type, operand_type);
 	EwWork W;
 	memset(&W, 0, sizeof(W));
-	const int rc = ewise_run(x, op, operand, operand_type, operand_len,
-				 margin, out_type, &W, out, warn);
+	const int rc = out_type == SVTGPU_LGL
+		? compare_run(x, operand_on_left ? svt_ew_mirror(op) : op,
+			      operand, operand_type, operand_len, margin, &W, out)
+		: ewise_run(x, op, operand, operand_type, operand_len, margin,
+			    out_type, &W, out, warn);
 	if (W.d_aux != NULL)
 		svt_free_async(W.d_aux, 0);
 	if (W.d_counts != NULL)

@@ -182,10 +182,13 @@ class DeviceSVT:
 
     # -- element-wise operations (new shard, no collective) ------------
     def ewise(self, op, operand=None, margin=0, operand_on_left=False):
-        """x * v, v * x, x / v (op "*" / "/") or a Math function ("abs",
-        "sign", "sqrt", "floor", "ceiling", "trunc", "log1p", "expm1") as a
-        new owning DeviceSVT with the same columns; see svtgpu_ewise() in
-        include/svtgpu.h.  margin 2 takes the per-column vector of the whole
+        """x * v, v * x, x / v (op "*" / "/"), a Math function ("abs",
+        "sign", "sqrt", "floor", "ceiling", "trunc", "log1p", "expm1"), a
+        comparison (">", ">=", "<", "<=", "==", "!=") or "is.na", "is.nan",
+        "is.infinite" as a new owning DeviceSVT with the same columns; see
+        svtgpu_ewise() in include/svtgpu.h.  Comparisons and the is.*
+        predicates give a "logical" result, without a value array when it
+        holds no NA.  margin 2 takes the per-column vector of the whole
         matrix (length nleaf_total, sliced to this shard's columns) or this
         shard's slice.  The result's `warnings` lists R's warnings."""
         code = N.EW_OPCODES.get(op)
@@ -193,7 +196,7 @@ class DeviceSVT:
             raise ValueError("unsupported element-wise operation %r" % (op,))
         vp, vt, vlen = None, 0, 0
         keep = None
-        if code in (N.EW_OPCODES["*"], N.EW_OPCODES["/"]):
+        if op in ("*", "/") + N.EW_COMPARE:
             a = np.asarray(operand).reshape(-1)
             if margin == 2 and a.size == self.nleaf_total and \
                     self.nleaf != self.nleaf_total:
@@ -213,7 +216,8 @@ class DeviceSVT:
         nnz, vtype = ctypes.c_int64(0), ctypes.c_int(0)
         N.check(N.lib().svtgpu_matrix_info(h, None, None, ctypes.byref(nnz),
                                            ctypes.byref(vtype), None))
-        type_ = {N.INT: "integer", N.DOUBLE: "double"}[vtype.value]
+        type_ = {N.LGL: "logical", N.INT: "integer",
+                 N.DOUBLE: "double"}[vtype.value]
         out = DeviceSVT(self.nrow, self.nleaf, nnz.value, type_, None, None,
                         None, leaf0=self.leaf0, nleaf_total=self.nleaf_total,
                         handle=h, owns_handle=True)

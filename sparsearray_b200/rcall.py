@@ -67,7 +67,8 @@ def registered_routines():
                  "C_svtgpu_release", "C_svtgpu_from_CSC", "C_svtgpu_to_CSC",
                  "C_svtgpu_set_cache",
                  "C_svtgpu_cache_stats", "C_svtgpu_Arith_SVT",
-                 "C_svtgpu_Math_SVT"):
+                 "C_svtgpu_Math_SVT", "C_svtgpu_Compare_SVT",
+                 "C_svtgpu_is_SVT"):
         n = ctypes.c_int(-1)
         p = L.rshim_lookup_call_routine(ctypes.byref(_info), name.encode(),
                                         ctypes.byref(n))

@@ -96,6 +96,9 @@ SEXP C_svtgpu_to_CSC(SEXP handle, SEXP as_ngCMatrix);
 SEXP C_svtgpu_Arith_SVT(SEXP x_dim, SEXP x_type, SEXP x_SVT, SEXP op, SEXP y,
 			SEXP margin, SEXP y_on_left);
 SEXP C_svtgpu_Math_SVT(SEXP x_dim, SEXP x_type, SEXP x_SVT, SEXP op);
+SEXP C_svtgpu_Compare_SVT(SEXP x_dim, SEXP x_type, SEXP x_SVT, SEXP op,
+			  SEXP y, SEXP margin, SEXP y_on_left);
+SEXP C_svtgpu_is_SVT(SEXP x_dim, SEXP x_type, SEXP x_SVT, SEXP fun);
 SEXP C_svtgpu_set_cache(SEXP on);
 SEXP C_svtgpu_cache_stats(void);
 SEXP C_get_num_procs(void);

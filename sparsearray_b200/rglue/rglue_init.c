@@ -68,6 +68,8 @@ static const R_CallMethodDef callMethods[] = {
 	CALLMETHOD_DEF(C_svtgpu_to_CSC, 2),
 	CALLMETHOD_DEF(C_svtgpu_Arith_SVT, 7),
 	CALLMETHOD_DEF(C_svtgpu_Math_SVT, 4),
+	CALLMETHOD_DEF(C_svtgpu_Compare_SVT, 7),
+	CALLMETHOD_DEF(C_svtgpu_is_SVT, 4),
 	CALLMETHOD_DEF(C_svtgpu_set_cache, 1),
 	CALLMETHOD_DEF(C_svtgpu_cache_stats, 0),
 	{NULL, NULL, 0}

@@ -224,6 +224,21 @@ class SVT_SparseArray:
     def __rtruediv__(self, other):
         return Arith(other, "/", self)   # refused: v / x
 
+    # -- Compare (x op v; `v < x` reaches x.__gt__(v)); see Compare().  No
+    # __eq__ / __ne__: SVT objects compare and hash by identity, so `==` and
+    # `!=` go through Compare() ----------------------------------------------
+    def __gt__(self, other):
+        return Compare(self, ">", other)
+
+    def __ge__(self, other):
+        return Compare(self, ">=", other)
+
+    def __lt__(self, other):
+        return Compare(self, "<", other)
+
+    def __le__(self, other):
+        return Compare(self, "<=", other)
+
 
 class ResidentSVT(SVT_SparseArray):
     """An SVT_SparseArray whose SVT already lives in HBM: `r_SVT` is the
@@ -337,7 +352,10 @@ def _ewise_result(ans, x):
     return _resident_like(x, handle, type_)
 
 
-def _arith_call(x, op, y, margin, y_on_left):
+_COMPARE_OPS = (">", ">=", "<", "<=", "==", "!=")
+
+
+def _arith_call(x, op, y, margin, y_on_left, entry="C_svtgpu_Arith_SVT"):
     if not isinstance(op, str):
         raise TypeError("'op' must be a single string")
     yv = _operand(y)
@@ -345,8 +363,8 @@ def _arith_call(x, op, y, margin, y_on_left):
              rshim.logical([int(y_on_left)])]
     try:
         ans, warns = rcall.SparseArray_Call(
-            "C_svtgpu_Arith_SVT", x.r_dim, x.r_type, x.r_SVT, temps[1], yv,
-            temps[2], temps[3])
+            entry, x.r_dim, x.r_type, x.r_SVT, temps[1], yv, temps[2],
+            temps[3])
     finally:
         for t in temps:
             t.release()
@@ -376,13 +394,67 @@ def Arith(e1, op, e2):
 def sweep(x, MARGIN, STATS, FUN="-"):
     """sweep(x, MARGIN, STATS, FUN) for FUN "*" or "/": STATS[i] applied to
     row i (MARGIN = 1) or STATS[j] to column j of a matrix (MARGIN = 2), as
-    `t(t(x) / sf)`.  FUN defaults to "-" as in R, which is refused (it would
-    fill the implicit zeros)."""
+    `t(t(x) / sf)`; a comparison FUN (">", ">=", "<", "<=", "==", "!=")
+    goes to Compare().  FUN defaults to "-" as in R, which is refused (it
+    would fill the implicit zeros)."""
     if not isinstance(x, SVT_SparseArray):
         raise TypeError("'x' must be an SVT_SparseArray")
     if MARGIN not in (1, 2):
         _wmsg_stop("'MARGIN' must be 1 or 2")
+    if FUN in _COMPARE_OPS:
+        return _arith_call(x, FUN, STATS, int(MARGIN), False,
+                           "C_svtgpu_Compare_SVT")
     return _arith_call(x, FUN, STATS, int(MARGIN), False)
+
+
+def Compare(e1, op, e2):
+    """`e1 op e2` for op ">", ">=", "<", "<=", "==" or "!=" where one side is
+    an SVT_SparseArray and the other a numeric scalar or a vector of length
+    nrow(x) (recycled along the first dimension, as in Arith()).  Admitted
+    only when `0 op v` is FALSE for every element of the operand, so the
+    implicit zeros stay FALSE (`x > 0`, `x >= 1`, `x == 3`, `x != 0`); any
+    NA or NaN operand is refused.  Served on the device: returns a new
+    ResidentSVT of type "logical" holding TRUE (and NA where x is NA or
+    NaN)."""
+    if isinstance(e1, SVT_SparseArray):
+        x, y, on_left = e1, e2, False
+    elif isinstance(e2, SVT_SparseArray):
+        x, y, on_left = e2, e1, True
+    else:
+        raise TypeError("one operand must be an SVT_SparseArray")
+    n = np.asarray(y).size
+    return _arith_call(x, op, y, 0 if n == 1 else 1, on_left,
+                       "C_svtgpu_Compare_SVT")
+
+
+def _is_call(x, fun):
+    if not isinstance(x, SVT_SparseArray):
+        raise TypeError("'x' must be an SVT_SparseArray")
+    t = rshim.string(fun)
+    try:
+        ans, warns = rcall.SparseArray_Call("C_svtgpu_is_SVT", x.r_dim,
+                                            x.r_type, x.r_SVT, t)
+    finally:
+        t.release()
+    r = _ewise_result(ans, x)
+    r.warnings = warns
+    return r
+
+
+def is_na(x):
+    """is.na(x): a new logical ResidentSVT, TRUE where x holds NA or NaN."""
+    return _is_call(x, "is.na")
+
+
+def is_nan(x):
+    """is.nan(x): TRUE where x holds a NaN that is not NA (never for integer
+    or logical x)."""
+    return _is_call(x, "is.nan")
+
+
+def is_infinite(x):
+    """is.infinite(x): TRUE where x holds Inf or -Inf."""
+    return _is_call(x, "is.infinite")
 
 
 def Math(x, op):

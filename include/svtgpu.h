@@ -271,6 +271,32 @@ int svtgpu_summarize(svtgpu_matrix *m, int opcode, int narm, double center,
 int svtgpu_rowstats_via_transpose(svtgpu_matrix *m, int opcode, int narm,
 				  double center, void *out, int *warn);
 
+/* ---- medians ----
+ * base R's median() of every dense column (svtgpu_colmedians; out[nleaf],
+ * host) or row (svtgpu_rowmedians; out[nrow], host, computed as column
+ * medians of the device transpose, which stays cached in m) as doubles,
+ * replacing the R-level colMedians() / rowMedians() methods
+ * (R/SparseArray-matrixStats.R:760-813).  A column holding NA or NaN gives
+ * NA_real_ unless narm; with narm they are removed and an empty remainder
+ * gives NA_real_.  Even counts give the correctly rounded midpoint of the
+ * two middle values; -Inf and +Inf as the middles give NaN.  Every result
+ * is exact (rules: svt_med_* in csrc/svt_semantics.h).  Logical input is
+ * 0 / 1, lacunar leaves hold ones.
+ * svtgpu_colmedians_dev(): result left in device memory (d_out[nleaf]),
+ * enqueued on `stream`; no sync.
+ * svtgpu_colmedians_selected(): how many leaves (rows) the last
+ * svtgpu_colmedians / svtgpu_rowmedians on m sent to exact selection, i.e.
+ * whose median the stored-value counts did not decide, and how many stored
+ * values the selection passes read in all (either pointer may be NULL).
+ * Only the host-result calls record these counts: svtgpu_colmedians_dev()
+ * does not synchronise and leaves them unchanged. */
+int svtgpu_colmedians(svtgpu_matrix *m, int narm, double *out);
+int svtgpu_colmedians_dev(svtgpu_matrix *m, int narm, double *d_out,
+			  void *stream);
+int svtgpu_rowmedians(svtgpu_matrix *m, int narm, double *out);
+int svtgpu_colmedians_selected(const svtgpu_matrix *m, int64_t *n_leaves,
+			       int64_t *n_reads);
+
 /* Two-stage form for column-sharded matrices (one shard per GPU/process):
  * accumulate() reduces this shard's leaves into a per-row state of
  * svtgpu_rowstats_state_len() doubles laid out as `nslots` arrays of nrow:

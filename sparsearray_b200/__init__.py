@@ -18,7 +18,7 @@ from .svt import (SVT_SparseArray, SVT_SparseMatrix, ResidentSVT, to_device,  # 
                   NA_REAL, is_na_real,
                   colSums, colMeans, colVars, colSds, colMins, colMaxs,
                   colRanges, colProds, colAnyNAs, colCountNAs, colAnys,
-                  colAlls, colSums2, colMeans2,
+                  colAlls, colSums2, colMeans2, colMedians, rowMedians,
                   rowSums, rowMeans, rowVars, rowSds, rowMins, rowMaxs,
                   rowRanges, rowAnyNAs, rowCountNAs, rowSums2, rowMoments,
                   rowProds, rowMeans2, rowAnys, rowAlls,

@@ -79,6 +79,11 @@ SIGNATURES = {
                                              _c.POINTER(_INT)]),
     "svtgpu_rowsum": (_INT, [_P, _P, _INT, _INT, _P, _c.POINTER(_INT)]),
     "svtgpu_colsum": (_INT, [_P, _P, _INT, _INT, _P, _c.POINTER(_INT)]),
+    "svtgpu_colmedians": (_INT, [_P, _INT, _P]),
+    "svtgpu_colmedians_dev": (_INT, [_P, _INT, _P, _P]),
+    "svtgpu_rowmedians": (_INT, [_P, _INT, _P]),
+    "svtgpu_colmedians_selected": (_INT, [_P, _c.POINTER(_I64),
+                                          _c.POINTER(_I64)]),
     "svtgpu_summarize_supported": (_INT, [_INT, _INT]),
     "svtgpu_summarize": (_INT, [_P, _INT, _INT, _DBL, _c.POINTER(_DBL),
                                 _c.POINTER(_INT)]),

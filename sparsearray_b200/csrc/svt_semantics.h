@@ -1004,4 +1004,121 @@ SVT_HD double svt_ew_dbl(int op, double x, int x_na, double v, uint32_t *fl)
 	return r;
 }
 
+/* ------------------------------------------------------------------------
+ * Medians (svtgpu_colmedians / svtgpu_rowmedians)
+ *
+ * Base R's median() of each dense column: NA_real_ when the column holds an
+ * NA or NaN and na.rm is FALSE (median.default returns x[NA_integer_]); with
+ * na.rm, NA and NaN are removed and nothing left gives NA_real_.  Otherwise
+ * the value at 0-based rank (n-1)/2 of the sorted column, or for even n the
+ * midpoint of the values at ranks n/2 - 1 and n/2.
+ *
+ * The implicit zeros (and stored zeros, +0 or -0) form one block in the
+ * middle of the sorted order: [negatives | zeros | positives].  The counts of
+ * stored negatives, positives and NA / NaN decide whether the middle ranks
+ * fall inside the zero block; only when they do not does a kernel select a
+ * stored value by rank, among the values of one sign ("side").
+ */
+#define SVT_MED_NA       0  /* the result is NA_real_ */
+#define SVT_MED_ZERO     1  /* the result is +0 */
+#define SVT_MED_SELECT   2  /* select the value at `rank` of `side` */
+
+#define SVT_MED_NEG      0
+#define SVT_MED_POS      1
+
+#define SVT_MED_2ND_NONE 0  /* odd count: the selected value is the median */
+#define SVT_MED_2ND_ZERO 1  /* midpoint of the selected value and 0 */
+#define SVT_MED_2ND_NEXT 2  /* midpoint of the selected value and the next
+			       larger stored nonzero value (either side) */
+
+typedef struct SvtMedPlan {
+	int kind;      /* SVT_MED_NA / _ZERO / _SELECT */
+	int side;      /* SVT_MED_NEG / _POS (SELECT only) */
+	int second;    /* SVT_MED_2ND_* (SELECT only) */
+	int64_t rank;  /* 0-based rank among the side's values, ascending */
+} SvtMedPlan;
+
+/* nrow: length of the column; nneg / npos: stored values < 0 / > 0; nna:
+   stored NA or NaN (stored zeros count in none of the three) */
+SVT_HD SvtMedPlan svt_med_plan(int64_t nrow, int64_t nneg, int64_t npos,
+			       int64_t nna, int narm)
+{
+	SvtMedPlan p;
+	p.kind = SVT_MED_NA;
+	p.side = SVT_MED_NEG;
+	p.second = SVT_MED_2ND_NONE;
+	p.rank = 0;
+	if (nna > 0 && !narm)
+		return p;
+	const int64_t n = nrow - nna;
+	if (n <= 0)
+		return p;
+	const int64_t z0 = nneg;                  /* first rank of the zeros */
+	const int64_t p0 = n - npos;              /* first rank of positives */
+	const int64_t lo = (n - 1) / 2, hi = n / 2;
+	if (lo >= z0 && hi < p0) {
+		p.kind = SVT_MED_ZERO;
+		return p;
+	}
+	p.kind = SVT_MED_SELECT;
+	if (lo < z0) {
+		p.side = SVT_MED_NEG;
+		p.rank = lo;
+		p.second = hi == lo ? SVT_MED_2ND_NONE
+			 : (hi < z0 || hi >= p0) ? SVT_MED_2ND_NEXT
+			 : SVT_MED_2ND_ZERO;
+	} else if (lo >= p0) {
+		p.side = SVT_MED_POS;
+		p.rank = lo - p0;
+		p.second = hi == lo ? SVT_MED_2ND_NONE : SVT_MED_2ND_NEXT;
+	} else {
+		/* lo is the last zero, hi the first positive */
+		p.side = SVT_MED_POS;
+		p.rank = 0;
+		p.second = SVT_MED_2ND_ZERO;
+	}
+	return p;
+}
+
+/* The midpoint of the two middle values, correctly rounded: (a + b) / 2
+ * when a + b is finite (halving is exact), a/2 + b/2 when a + b overflows
+ * for finite a and b (base R's mean() sums in long double and gets the
+ * same).  -Inf and +Inf give NaN (never NA); a zero result is +0. */
+SVT_HD double svt_med_mid(double a, double b)
+{
+	const double s = a + b;
+	if (svt_isnan(s))
+		return svt_nan();
+	if (!svt_isfinite(s) && svt_isfinite(a) && svt_isfinite(b))
+		return a / 2.0 + b / 2.0;
+	return s / 2.0 + 0.0;
+}
+
+/* Order-preserving unsigned keys.  int32: NA_integer_ (INT_MIN) is not a
+ * key (returns 0); every other value maps to x ^ 0x80000000, so keys of
+ * non-NA values are >= 1.  double: NaN (NA included) is not a key; -x sorts
+ * before +x, -0 before +0 (the kernels never select a zero). */
+SVT_HD int svt_med_key_i32(int32_t x, uint32_t *key)
+{
+	*key = (uint32_t) x ^ 0x80000000u;
+	return x != SVT_NA_INT;
+}
+
+SVT_HD int32_t svt_med_unkey_i32(uint32_t key)
+{
+	return (int32_t) (key ^ 0x80000000u);
+}
+
+SVT_HD int svt_med_key_f64(double x, uint64_t *key)
+{
+	const uint64_t u = svt_d2u(x);
+	*key = (u >> 63) ? ~u : (u | 0x8000000000000000ULL);
+	return !svt_isnan(x);
+}
+
+SVT_HD double svt_med_unkey_f64(uint64_t key)
+{
+	return svt_u2d((key >> 63) ? (key & 0x7FFFFFFFFFFFFFFFULL) : ~key);
+}
+
 #endif  /* SVT_SEMANTICS_H */

@@ -63,6 +63,9 @@ struct svtgpu_matrix {
 	int8_t *d_vals8;     /* nnz + SVT_COMPACT_PAD, or NULL */
 	int compact_state;   /* SVT_COMPACT_NONE / _BUILT / _INELIGIBLE */
 	int compact_uses;    /* eligible statistic calls seen while NONE */
+	int64_t med_selected;  /* leaves sent to selection by the last
+				  svtgpu_colmedians / svtgpu_rowmedians */
+	int64_t med_select_reads;  /* values its selection passes read */
 
 	svtgpu_timings tm;
 };

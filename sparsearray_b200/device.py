@@ -260,6 +260,38 @@ class DeviceSVT:
             _ptr(warn), _stream_ptr()))
         return out, warn
 
+    def colmedians(self, na_rm=False, out=None):
+        """colMedians() of the local columns as doubles, left on the
+        device (svtgpu_colmedians_dev; no collective)."""
+        if out is None:
+            out = torch.empty(self.nleaf, device="cuda", dtype=torch.float64)
+        N.check(N.lib().svtgpu_colmedians_dev(self._h, int(na_rm), _ptr(out),
+                                              _stream_ptr()))
+        return out
+
+    def rowmedians(self, na_rm=False):
+        """rowMedians() as doubles on the host, through the device transpose
+        (cached in the handle).  Only for a shard that holds every column:
+        a row median does not compose across column shards."""
+        if self.nleaf != self.nleaf_total:
+            raise ValueError("rowmedians() needs every column of the matrix "
+                             "(this shard holds %d of %d): a row median does "
+                             "not compose across column shards"
+                             % (self.nleaf, self.nleaf_total))
+        out = np.zeros(self.nrow, dtype=np.float64)
+        N.check(N.lib().svtgpu_rowmedians(
+            self._h, int(na_rm), out.ctypes.data_as(ctypes.c_void_p)))
+        return out
+
+    def median_selected(self):
+        """(columns or rows sent to exact selection, stored values its passes
+        read) by the last host-result median call on this handle
+        (svtgpu_colmedians_selected)."""
+        n, r = ctypes.c_int64(0), ctypes.c_int64(0)
+        N.check(N.lib().svtgpu_colmedians_selected(self._h, ctypes.byref(n),
+                                                   ctypes.byref(r)))
+        return n.value, r.value
+
     # -- whole-array summaries (host scalars; sum()/mean()/var()/range()) --
     def summarize(self, op, na_rm=False, center=None):
         """C_summarize_SVT over the local shard: (values, warn) on the host;

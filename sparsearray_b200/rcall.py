@@ -63,6 +63,7 @@ def registered_routines():
                  "C_crossprod1_SVT", "C_matmul_SVT_mat",
                  "C_summarize_SVT", "C_rowsum_SVT", "C_colsum_SVT",
                  "C_rowMoments_SVT", "C_rowStatsT_SVT",
+                 "C_colMedians_SVT", "C_rowMedians_SVT",
                  "C_svtgpu_last_timings", "C_svtgpu_resident_SVT",
                  "C_svtgpu_release", "C_svtgpu_from_CSC", "C_svtgpu_to_CSC",
                  "C_svtgpu_set_cache",

@@ -86,6 +86,10 @@ SEXP C_rowMoments_SVT(SEXP x_dim, SEXP x_dimnames, SEXP x_type, SEXP x_SVT,
 SEXP C_rowStatsT_SVT(SEXP x_dim, SEXP x_dimnames, SEXP x_type, SEXP x_SVT,
 		     SEXP x_na_background, SEXP op, SEXP na_rm, SEXP center,
 		     SEXP dims);
+SEXP C_colMedians_SVT(SEXP x_dim, SEXP x_dimnames, SEXP x_type, SEXP x_SVT,
+		      SEXP na_rm);
+SEXP C_rowMedians_SVT(SEXP x_dim, SEXP x_dimnames, SEXP x_type, SEXP x_SVT,
+		      SEXP na_rm);
 SEXP C_svtgpu_last_timings(void);
 SEXP C_svtgpu_resident_SVT(SEXP x_dim, SEXP x_type, SEXP x_SVT);
 SEXP C_svtgpu_release(SEXP handle);

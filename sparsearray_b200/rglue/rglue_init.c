@@ -61,6 +61,8 @@ static const R_CallMethodDef callMethods[] = {
 	CALLMETHOD_DEF(C_matmul_SVT_mat, 5),
 	CALLMETHOD_DEF(C_rowMoments_SVT, 5),
 	CALLMETHOD_DEF(C_rowStatsT_SVT, 9),
+	CALLMETHOD_DEF(C_colMedians_SVT, 5),
+	CALLMETHOD_DEF(C_rowMedians_SVT, 5),
 	CALLMETHOD_DEF(C_svtgpu_last_timings, 0),
 	CALLMETHOD_DEF(C_svtgpu_resident_SVT, 3),
 	CALLMETHOD_DEF(C_svtgpu_release, 1),

@@ -337,3 +337,66 @@ SEXP C_rowMoments_SVT(SEXP x_dim, SEXP x_dimnames, SEXP x_type, SEXP x_SVT,
 	UNPROTECT(1);
 	return ans;
 }
+
+/* colMedians() / rowMedians() of a matrix: one double per column / row
+   (svtgpu_colmedians / svtgpu_rowmedians) */
+static SEXP medians_SVT(SEXP x_dim, SEXP x_dimnames, SEXP x_type, SEXP x_SVT,
+			SEXP na_rm, int rows, const char *fun)
+{
+	SEXPTYPE x_Rtype = rglue_get_and_check_Rtype(x_type, fun, "x_type");
+	if (!(IS_LOGICAL(na_rm) && LENGTH(na_rm) == 1))
+		error("'na.rm' must be TRUE or FALSE");
+	int narm = LOGICAL(na_rm)[0];
+	const char *what = rows ? "rowMedians()" : "colMedians()";
+	check_gpu_input(x_Rtype, 0, what);
+	const int *dim = INTEGER(x_dim);
+	int ndim = LENGTH(x_dim);
+	if (ndim != 2)
+		error("%s: only matrices (2-dimensional objects) are supported; "
+		      "'x' has %d dimensions", what, ndim);
+	const int nout = dim[rows ? 0 : 1], nin = dim[rows ? 1 : 0];
+	SEXP ans = PROTECT(NEW_NUMERIC(nout));
+	propagate_dimnames(ans, x_dimnames, rows ? 0 : 1, 1);
+	if (nout == 0) {
+		UNPROTECT(1);
+		return ans;
+	}
+	if (nin == 0) {
+		/* every median is over an empty vector */
+		SvtMedPlan p = svt_med_plan(0, 0, 0, 0, narm);
+		for (int i = 0; i < nout; i++)
+			REAL(ans)[i] = p.kind == SVT_MED_NA ? NA_REAL : 0.0;
+		UNPROTECT(1);
+		return ans;
+	}
+	rglue_input in;
+	rglue_acquire(x_SVT, dim, ndim, x_Rtype, rows, 1, &in);
+	int rc = rows ? svtgpu_rowmedians(in.m, narm, REAL(ans))
+		      : svtgpu_colmedians(in.m, narm, REAL(ans));
+	rglue_done(&in, fun);
+	if (rc != SVTGPU_OK)
+		rglue_fail(rc, rows ? "svtgpu_rowmedians" : "svtgpu_colmedians");
+	UNPROTECT(1);
+	return ans;
+}
+
+/* --- .Call ENTRY POINT (extension) ---
+ * colMedians() of a 2-D SVT, which the reference computes in R
+ * (R/SparseArray-matrixStats.R:760-813): base R's median() of every dense
+ * column as a double vector, named by the column names. */
+SEXP C_colMedians_SVT(SEXP x_dim, SEXP x_dimnames, SEXP x_type, SEXP x_SVT,
+		      SEXP na_rm)
+{
+	return medians_SVT(x_dim, x_dimnames, x_type, x_SVT, na_rm, 0,
+			   "C_colMedians_SVT");
+}
+
+/* --- .Call ENTRY POINT (extension) ---
+ * rowMedians() of a 2-D SVT: the column medians of the device transpose,
+ * which stays cached in a resident handle. */
+SEXP C_rowMedians_SVT(SEXP x_dim, SEXP x_dimnames, SEXP x_type, SEXP x_SVT,
+		      SEXP na_rm)
+{
+	return medians_SVT(x_dim, x_dimnames, x_type, x_SVT, na_rm, 1,
+			   "C_rowMedians_SVT");
+}

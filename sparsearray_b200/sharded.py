@@ -50,6 +50,12 @@ def colVars(x, na_rm=False, center=None):
     return S.colVars(x, na_rm=na_rm, center=center)
 
 
+def colMedians(x, na_rm=False):
+    """Final per shard.  There is no sharded rowMedians(): a row median does
+    not compose from the medians of column pieces."""
+    return S.colMedians(x, na_rm=na_rm)
+
+
 def rowSums(x, na_rm=False, group=None):
     return _allreduce_sum(S.rowSums(x, na_rm=na_rm), group)
 

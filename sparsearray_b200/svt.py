@@ -804,6 +804,30 @@ def rowSds(x, na_rm=False, center=None, dims=1, useNames=None):
         return _keep_na(v, np.sqrt(v))
 
 
+def _medians(entry, x, na_rm, useNames):
+    if not isinstance(x, SVT_SparseArray):
+        raise TypeError("'x' must be an SVT_SparseArray")
+    if not isinstance(na_rm, (bool, np.bool_)):
+        _wmsg_stop("'na.rm' must be TRUE or FALSE")
+    useNames = _normarg_useNames(useNames)
+    temps = [rshim.logical([int(na_rm)])]
+    args = [x.r_dim, x.r_dimnames if useNames else None, x.r_type, x.r_SVT,
+            temps[0]]
+    return _call(entry, args, temps)
+
+
+def colMedians(x, na_rm=False, useNames=None):
+    """Base R's median() of every column of a matrix, as doubles (the
+    reference's colMedians() method, R/SparseArray-matrixStats.R:760-785)."""
+    return _medians("C_colMedians_SVT", x, na_rm, useNames)
+
+
+def rowMedians(x, na_rm=False, useNames=None):
+    """Base R's median() of every row of a matrix, as doubles (:787-813);
+    computed on the device transpose, which a resident handle keeps."""
+    return _medians("C_rowMedians_SVT", x, na_rm, useNames)
+
+
 def rowMoments(x, na_rm=False):
     """Extension: rowMeans + rowVars(center=NULL) in ONE pass over the SVT
     (the reference needs three C_rowStats_SVT passes).  Returns (mean, var)."""

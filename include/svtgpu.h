@@ -414,6 +414,27 @@ int svtgpu_ewise(svtgpu_matrix *x, int op, const void *operand,
 		 int operand_type, int64_t operand_len, int margin,
 		 int operand_on_left, svtgpu_matrix **out, int *warn);
 
+/* ---- element-wise operations between two matrices ----
+ * `x op y` for two device matrices of the same geometry (nrow and nleaf),
+ * with base R's dense semantics of `as.matrix(x) op as.matrix(y)`; the
+ * implicit zeros stay 0 / FALSE, so op is one of SVTGPU_EW_ADD, SUB, MUL,
+ * AND, OR, GT, LT, NE (`/`, `^`, `%%`, `%/%`, `==`, `>=`, `<=` would fill
+ * them and are refused with SVTGPU_ERR_ARG).  *out is a NEW matrix of x's
+ * geometry with ascending offsets in every leaf and no cached knowledge;
+ * computed zeros (and FALSE) are dropped.  Arith gives integer unless a side
+ * is double (logical op logical gives integer); Logic and Compare give a
+ * logical result stored as for svtgpu_ewise()'s comparisons.  x and y may be
+ * the same matrix.  *warn: SVTGPU_EW_WARN_INT_OVERFLOW.  Geometry, types and
+ * op are checked before a device is asked for; out of memory returns
+ * SVTGPU_ERR_NOMEM with nothing left allocated.  Rules: svt_ew2_* in
+ * csrc/svt_semantics.h. */
+#define SVTGPU_EW_ADD       3
+#define SVTGPU_EW_SUB       4
+#define SVTGPU_EW_AND      41
+#define SVTGPU_EW_OR       42
+int svtgpu_ewise2(svtgpu_matrix *x, svtgpu_matrix *y, int op,
+		  svtgpu_matrix **out, int *warn);
+
 /* ---- synthetic data (benchmark inputs, generated in HBM) ----
  * Counter-based, so any leaf can be regenerated anywhere: with
  *   h  = mix64(seed + (cell + 1) * 0x9E3779B97F4A7C15),  cell = leaf*nrow + i

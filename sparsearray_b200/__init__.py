@@ -12,7 +12,7 @@ Importing the package never touches CUDA; the first call does, and fails
 loudly when the extension or a device is missing (there is no CPU fallback).
 """
 from .svt import (SVT_SparseArray, SVT_SparseMatrix, ResidentSVT, to_device,  # noqa: F401
-                  from_csc, to_csc, Arith, Math, sweep, Compare,
+                  from_csc, to_csc, Arith, Math, sweep, Compare, Logic,
                   is_na, is_nan, is_infinite,
                   RArray, NA_INTEGER,
                   NA_REAL, is_na_real,

@@ -108,6 +108,7 @@ SIGNATURES = {
     "svtgpu_exclusive_scan": (_INT, [_P, _I64, _P, _P]),
     "svtgpu_ewise": (_INT, [_P, _INT, _P, _INT, _I64, _INT, _INT,
                             _c.POINTER(_P), _c.POINTER(_INT)]),
+    "svtgpu_ewise2": (_INT, [_P, _P, _INT, _c.POINTER(_P), _c.POINTER(_INT)]),
 }
 
 # element-wise opcodes (SVTGPU_EW_*) and warning bits
@@ -116,6 +117,9 @@ EW_OPCODES = {"*": 1, "/": 2, "abs": 11, "sign": 12, "sqrt": 13, "floor": 14,
               ">": 21, ">=": 22, "<": 23, "<=": 24, "==": 25, "!=": 26,
               "is.na": 31, "is.nan": 32, "is.infinite": 33}
 EW_COMPARE = (">", ">=", "<", "<=", "==", "!=")
+# opcodes of svtgpu_ewise2 (two matrices): "*", ">", "<", "!=" as above
+EW2_OPCODES = {"+": 3, "-": 4, "*": 1, "&": 41, "|": 42, ">": 21, "<": 23,
+               "!=": 26}
 EW_WARN_INT_OVERFLOW, EW_WARN_NAN = 1, 2
 EW_WARNINGS = ((EW_WARN_INT_OVERFLOW, "NAs produced by integer overflow"),
                (EW_WARN_NAN, "NaNs produced"))

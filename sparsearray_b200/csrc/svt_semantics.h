@@ -1005,6 +1005,184 @@ SVT_HD double svt_ew_dbl(int op, double x, int x_na, double v, uint32_t *fl)
 }
 
 /* ------------------------------------------------------------------------
+ * Element-wise operations between two SVTs (svtgpu_ewise2)
+ *
+ * `x op y` of two arrays of the same dimensions, as base R computes
+ * `as.matrix(x) op as.matrix(y)` (src/main/arithmetic.c: R_integer_plus(),
+ * R_integer_minus(), R_integer_times(), real_binary(); relop.c; logic.c),
+ * zeros dropped.  Only operators that map two zeros to 0 / FALSE are
+ * admitted.  An entry stored on one side only meets an implicit zero on the
+ * other (the value 0, never NA), so one rule per operator serves "x only",
+ * "y only" and "both".  The svt_ew2_* opcodes are not opcodes of
+ * svt_ew_check(): the scalar path keeps refusing them.
+ */
+SVT_HD int svt_ew2_is_arith(int op)
+{
+	return op == SVTGPU_EW_ADD || op == SVTGPU_EW_SUB || op == SVTGPU_EW_MUL;
+}
+
+SVT_HD int svt_ew2_is_logic(int op)
+{
+	return op == SVTGPU_EW_AND || op == SVTGPU_EW_OR;
+}
+
+SVT_HD int svt_ew2_is_compare(int op)
+{
+	return op == SVTGPU_EW_GT || op == SVTGPU_EW_LT || op == SVTGPU_EW_NE;
+}
+
+SVT_HD int svt_ew2_admitted(int op)
+{
+	return svt_ew2_is_arith(op) || svt_ew2_is_logic(op) ||
+	       svt_ew2_is_compare(op);
+}
+
+SVT_HD const char *svt_ew2_opname(int op)
+{
+	switch (op) {
+	    case SVTGPU_EW_ADD: return "+";
+	    case SVTGPU_EW_SUB: return "-";
+	    case SVTGPU_EW_MUL: return "*";
+	    case SVTGPU_EW_AND: return "&";
+	    case SVTGPU_EW_OR:  return "|";
+	    case SVTGPU_EW_GT:  return ">";
+	    case SVTGPU_EW_LT:  return "<";
+	    case SVTGPU_EW_NE:  return "!=";
+	}
+	return "?";
+}
+
+/* "+", "-", "*", "&", "|", ">", "<", "!=" -> opcode; any other name -> 0 */
+SVT_HD int svt_ew2_opcode(const char *name)
+{
+	const int ops[8] = { SVTGPU_EW_ADD, SVTGPU_EW_SUB, SVTGPU_EW_MUL,
+			     SVTGPU_EW_AND, SVTGPU_EW_OR, SVTGPU_EW_GT,
+			     SVTGPU_EW_LT, SVTGPU_EW_NE };
+	for (int k = 0; k < 8; k++)
+		if (svt_ew_streq(name, svt_ew2_opname(ops[k])))
+			return ops[k];
+	return 0;
+}
+
+/* Arith: integer unless a side is double (logical op logical is integer);
+   Logic and Compare: logical */
+SVT_HD int svt_ew2_result_type(int op, int x_type, int y_type)
+{
+	if (!svt_ew2_is_arith(op))
+		return SVTGPU_LGL;
+	return (x_type == SVTGPU_DOUBLE || y_type == SVTGPU_DOUBLE)
+		? SVTGPU_DOUBLE : SVTGPU_INT;
+}
+
+/* The R error message for an operator svt_ew2_opcode() does not admit
+ * (host only): what the implicit zeros would become, or the list of the
+ * operators served. */
+static inline void svt_ew2_refusal_message(const char *opname, char *buf,
+					   size_t len)
+{
+	const char *zeros = NULL;
+	char cmp[32];
+	if (svt_ew_streq(opname, "/"))
+		zeros = "NaN (0 / 0)";
+	else if (svt_ew_streq(opname, "^"))
+		zeros = "1 (0 ^ 0)";
+	else if (svt_ew_streq(opname, "%%") || svt_ew_streq(opname, "%/%"))
+		zeros = "NA (0 %% 0, 0 %/% 0)";
+	else if (svt_ew_streq(opname, "==") || svt_ew_streq(opname, ">=") ||
+		 svt_ew_streq(opname, "<="))
+		zeros = (snprintf(cmp, sizeof(cmp), "TRUE (0 %s 0)", opname),
+			 cmp);
+	if (zeros != NULL)
+		snprintf(buf, len, "operator \"%s\" between two SparseArray "
+			 "objects is not supported on the GPU path: the implicit "
+			 "zeros of the result would become %s", opname, zeros);
+	else
+		snprintf(buf, len, "operator \"%s\" between two SparseArray "
+			 "objects is not supported on the GPU path (supported: "
+			 "\"+\", \"-\", \"*\", \"&\", \"|\", \">\", \"<\", \"!=\")",
+			 opname);
+}
+
+/* Integer result of "+", "-", "*": NA_integer_ on either side gives NA; the
+ * result is computed in 64 bits and one outside (-2^31, 2^31) gives NA with
+ * the overflow warning (R_integer_plus(), R_integer_minus(),
+ * R_integer_times()). */
+SVT_HD int32_t svt_ew2_int(int op, int32_t x, int32_t y, uint32_t *fl)
+{
+	if (x == SVT_NA_INT || y == SVT_NA_INT)
+		return SVT_NA_INT;
+	const int64_t a = x, b = y;
+	const int64_t z = op == SVTGPU_EW_ADD ? a + b
+			: op == SVTGPU_EW_SUB ? a - b : a * b;
+	if (z > INT32_MAX || z <= INT32_MIN) {
+		*fl |= SVTGPU_EW_WARN_INT_OVERFLOW;
+		return SVT_NA_INT;
+	}
+	return (int32_t) z;
+}
+
+/* Double result of "+", "-", "*".  x_na / y_na: the operand is NA
+ * (NA_integer_ or R_IsNA()).  Written out rather than left to the FPU,
+ * whose choice among NaN operands differs between host and GPU: an NA or
+ * NaN operand passes through with its own bits, x's before y's (an integer
+ * NA as NA_real_; "-" does not negate a NaN); a NaN made from other values
+ * (Inf - Inf, Inf * 0) is the canonical quiet NaN.  No contraction. */
+SVT_HD double svt_ew2_dbl(int op, double x, int x_na, double y, int y_na)
+{
+	if (svt_isnan(x))
+		return x;
+	if (x_na)
+		return svt_na_real();
+	if (svt_isnan(y))
+		return y;
+	if (y_na)
+		return svt_na_real();
+	double r;
+#ifdef __CUDA_ARCH__
+	r = op == SVTGPU_EW_ADD ? __dadd_rn(x, y)
+	  : op == SVTGPU_EW_SUB ? __dsub_rn(x, y) : __dmul_rn(x, y);
+#else
+	r = op == SVTGPU_EW_ADD ? x + y : op == SVTGPU_EW_SUB ? x - y : x * y;
+#endif
+	return svt_isnan(r) ? svt_nan() : r;
+}
+
+/* Logic and Compare: SVT_CMP_TRUE, SVT_CMP_NA or SVT_CMP_DROP (FALSE).
+ * Logic: a nonzero value is TRUE, NA or NaN is NA; "&" is FALSE when a side
+ * is FALSE, "|" TRUE when a side is TRUE, otherwise NA wins.  Compare: an
+ * int32 is compared as a double (exact); NA or NaN on a side gives NA. */
+SVT_HD int svt_ew2_lgl(int op, double x, int x_na, double y, int y_na)
+{
+	const int xn = x_na || svt_isnan(x), yn = y_na || svt_isnan(y);
+	if (svt_ew2_is_logic(op)) {
+		const int xt = xn ? SVT_CMP_NA
+			: x != 0.0 ? SVT_CMP_TRUE : SVT_CMP_DROP;
+		const int yt = yn ? SVT_CMP_NA
+			: y != 0.0 ? SVT_CMP_TRUE : SVT_CMP_DROP;
+		if (op == SVTGPU_EW_AND) {
+			if (xt == SVT_CMP_DROP || yt == SVT_CMP_DROP)
+				return SVT_CMP_DROP;
+			return (xt == SVT_CMP_NA || yt == SVT_CMP_NA)
+				? SVT_CMP_NA : SVT_CMP_TRUE;
+		}
+		if (xt == SVT_CMP_TRUE || yt == SVT_CMP_TRUE)
+			return SVT_CMP_TRUE;
+		return (xt == SVT_CMP_NA || yt == SVT_CMP_NA)
+			? SVT_CMP_NA : SVT_CMP_DROP;
+	}
+	if (xn || yn)
+		return SVT_CMP_NA;
+	bool r;
+	switch (op) {
+	    case SVTGPU_EW_GT: r = x >  y; break;
+	    case SVTGPU_EW_LT: r = x <  y; break;
+	    case SVTGPU_EW_NE: r = x != y; break;
+	    default:           return SVT_CMP_NA;
+	}
+	return r ? SVT_CMP_TRUE : SVT_CMP_DROP;
+}
+
+/* ------------------------------------------------------------------------
  * Medians (svtgpu_colmedians / svtgpu_rowmedians)
  *
  * Base R's median() of each dense column: NA_real_ when the column holds an

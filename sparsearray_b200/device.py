@@ -224,6 +224,34 @@ class DeviceSVT:
         out.warnings = [msg for bit, msg in N.EW_WARNINGS if warn.value & bit]
         return out
 
+    def ewise_svt(self, op, other):
+        """`self op other` ("+", "-", "*", "&", "|", ">", "<", "!=") of two
+        shards of the same column plan (same rows and columns) as a new
+        owning DeviceSVT; see svtgpu_ewise2() in include/svtgpu.h.  Logic
+        and Compare give a "logical" result.  The result's `warnings` lists
+        R's warnings."""
+        code = N.EW2_OPCODES.get(op)
+        if code is None:
+            raise ValueError("unsupported operation between two matrices %r"
+                             % (op,))
+        if (self.nrow, self.nleaf, self.leaf0) != \
+                (other.nrow, other.nleaf, other.leaf0):
+            raise ValueError("the shards cover different rows or columns")
+        h = ctypes.c_void_p()
+        warn = ctypes.c_int(0)
+        N.check(N.lib().svtgpu_ewise2(self._h, other._h, code,
+                                      ctypes.byref(h), ctypes.byref(warn)))
+        nnz, vtype = ctypes.c_int64(0), ctypes.c_int(0)
+        N.check(N.lib().svtgpu_matrix_info(h, None, None, ctypes.byref(nnz),
+                                           ctypes.byref(vtype), None))
+        type_ = {N.LGL: "logical", N.INT: "integer",
+                 N.DOUBLE: "double"}[vtype.value]
+        out = DeviceSVT(self.nrow, self.nleaf, nnz.value, type_, None, None,
+                        None, leaf0=self.leaf0, nleaf_total=self.nleaf_total,
+                        handle=h, owns_handle=True)
+        out.warnings = [msg for bit, msg in N.EW_WARNINGS if warn.value & bit]
+        return out
+
     def download(self):
         """(leaf_ptr, offs, vals) of the shard on the host (vals None when
         the shard stores no values)."""

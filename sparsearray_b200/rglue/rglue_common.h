@@ -103,6 +103,8 @@ SEXP C_svtgpu_Math_SVT(SEXP x_dim, SEXP x_type, SEXP x_SVT, SEXP op);
 SEXP C_svtgpu_Compare_SVT(SEXP x_dim, SEXP x_type, SEXP x_SVT, SEXP op,
 			  SEXP y, SEXP margin, SEXP y_on_left);
 SEXP C_svtgpu_is_SVT(SEXP x_dim, SEXP x_type, SEXP x_SVT, SEXP fun);
+SEXP C_svtgpu_Ops_SVT_SVT(SEXP x_dim, SEXP x_type, SEXP x_SVT, SEXP op,
+			  SEXP y_dim, SEXP y_type, SEXP y_SVT);
 SEXP C_svtgpu_set_cache(SEXP on);
 SEXP C_svtgpu_cache_stats(void);
 SEXP C_get_num_procs(void);

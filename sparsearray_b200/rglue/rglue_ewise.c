@@ -18,8 +18,12 @@
  *       `0 op y` is FALSE for every element of y
  *   C_svtgpu_is_SVT(x_dim, x_type, x_SVT, fun)
  *       fun "is.na", "is.nan" or "is.infinite"
+ *   C_svtgpu_Ops_SVT_SVT(x_dim, x_type, x_SVT, op, y_dim, y_type, y_SVT)
+ *       `x op y` of two SVTs (or handles) of identical dimensions, op "+",
+ *       "-", "*", "&", "|", ">", "<" or "!="
  *
- * All return list(handle, type); Compare and is.* give type "logical".  Every refusal (an operation that would
+ * All return list(handle, type); Compare, Logic and is.* give type
+ * "logical".  Every refusal (an operation that would
  * turn the implicit zeros into something else, a bad operand) is raised
  * before the device is touched; the input is never modified.  The warnings
  * carry R's wording.
@@ -174,4 +178,74 @@ SEXP C_svtgpu_is_SVT(SEXP x_dim, SEXP x_type, SEXP x_SVT, SEXP fun)
 		       0, 0, -1);
 	return run(x_dim, Rtype, x_SVT, code_op, NULL, 0, 0, 0, 0,
 		   "C_svtgpu_is_SVT");
+}
+
+/* --- .Call ENTRY POINT (extension) ---
+ * `x op y` between two SVT_SparseArray objects (the Arith, Logic and Compare
+ * methods with two SparseArray operands).  Order matters, as in
+ * C_crossprod2_SVT_SVT: every R error is raised while no per-call device
+ * matrix is held; y is indexed (or taken as a handle) before x is acquired
+ * and uploaded outside the device cache afterwards, so acquiring y can never
+ * free the x just taken from the cache; the same SVT on both sides is
+ * uploaded once. */
+SEXP C_svtgpu_Ops_SVT_SVT(SEXP x_dim, SEXP x_type, SEXP x_SVT, SEXP op,
+			  SEXP y_dim, SEXP y_type, SEXP y_SVT)
+{
+	const char *opname = get_op(op);
+	const int code_op = svt_ew2_opcode(opname);
+	if (code_op == 0) {
+		char msg[512];
+		svt_ew2_refusal_message(opname, msg, sizeof(msg));
+		error("%s", msg);
+	}
+	const char *fun = "C_svtgpu_Ops_SVT_SVT";
+	const SEXPTYPE x_Rtype = get_x_type(x_type, x_dim, fun, opname);
+	const SEXPTYPE y_Rtype = get_x_type(y_type, y_dim, fun, opname);
+	const int ndim = LENGTH(x_dim);
+	if (LENGTH(y_dim) != ndim ||
+	    memcmp(INTEGER(x_dim), INTEGER(y_dim), sizeof(int) * ndim) != 0)
+		error("non-conformable arrays");
+	const int *dim = INTEGER(x_dim);
+	rglue_input inx, iny;
+	const int same = y_SVT == x_SVT && y_Rtype == x_Rtype;
+	const int y_is_handle = TYPEOF(y_SVT) == EXTPTRSXP;
+	svt_leaf_index iy;
+	if (!same && y_is_handle)
+		rglue_acquire(y_SVT, dim, ndim, y_Rtype, 1, 1, &iny);
+	else if (!same)
+		svt_index_leaves(y_SVT, dim, ndim, y_Rtype, &iy);
+	rglue_acquire(x_SVT, dim, ndim, x_Rtype, 1, 1, &inx);
+	if (same) {
+		iny = inx;
+	} else if (!y_is_handle) {
+		memset(&iny, 0, sizeof(iny));
+		const int rcy = svt_upload_leaves(&iy, y_Rtype, 1, 1, &iny.m,
+						  &iny.flatten_ms);
+		iny.t_ready = rglue_now_ms();
+		if (rcy != SVTGPU_OK) {
+			rglue_done(&inx, fun);
+			rglue_fail(rcy, "svt_upload_leaves");
+		}
+	}
+	svtgpu_matrix *out = NULL;
+	int warn = 0;
+	const int rc = svtgpu_ewise2(inx.m, iny.m, code_op, &out, &warn);
+	/* the result is a new matrix: never the cached or a handle's one */
+	if (!same)
+		rglue_done(&iny, "C_svtgpu_Ops_SVT_SVT (y)");
+	rglue_done(&inx, fun);
+	if (rc != SVTGPU_OK)
+		rglue_fail(rc, "svtgpu_ewise2");
+	rglue_record_timings(out, 0.0);
+	int out_type = 0;
+	svtgpu_matrix_info(out, NULL, NULL, NULL, &out_type, NULL);
+	SEXP ans = PROTECT(NEW_LIST(2));
+	SET_VECTOR_ELT(ans, 0, rglue_make_handle(out));
+	SET_VECTOR_ELT(ans, 1, mkString(out_type == SVTGPU_DOUBLE ? "double"
+					: out_type == SVTGPU_LGL ? "logical"
+								  : "integer"));
+	if (warn & SVTGPU_EW_WARN_INT_OVERFLOW)
+		warning("NAs produced by integer overflow");
+	UNPROTECT(1);
+	return ans;
 }

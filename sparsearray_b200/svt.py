@@ -224,6 +224,32 @@ class SVT_SparseArray:
     def __rtruediv__(self, other):
         return Arith(other, "/", self)   # refused: v / x
 
+    # `x + y`, `x - y` need two SVTs; `x + 1` reaches Arith()'s refusal
+    def __add__(self, other):
+        return Arith(self, "+", other)
+
+    def __radd__(self, other):
+        return Arith(other, "+", self)
+
+    def __sub__(self, other):
+        return Arith(self, "-", other)
+
+    def __rsub__(self, other):
+        return Arith(other, "-", self)
+
+    # -- Logic between two SVTs; see Logic() --------------------------------
+    def __and__(self, other):
+        return Logic(self, "&", other)
+
+    def __rand__(self, other):
+        return Logic(other, "&", self)
+
+    def __or__(self, other):
+        return Logic(self, "|", other)
+
+    def __ror__(self, other):
+        return Logic(other, "|", self)
+
     # -- Compare (x op v; `v < x` reaches x.__gt__(v)); see Compare().  No
     # __eq__ / __ne__: SVT objects compare and hash by identity, so `==` and
     # `!=` go through Compare() ----------------------------------------------
@@ -373,6 +399,28 @@ def _arith_call(x, op, y, margin, y_on_left, entry="C_svtgpu_Arith_SVT"):
     return r
 
 
+def _ops2_call(e1, op, e2):
+    """`e1 op e2` of two SVT_SparseArray objects through
+    C_svtgpu_Ops_SVT_SVT; dimnames from e1, or from e2 when e1 has none."""
+    if not isinstance(op, str):
+        raise TypeError("'op' must be a single string")
+    t = rshim.string(op)
+    try:
+        ans, warns = rcall.SparseArray_Call(
+            "C_svtgpu_Ops_SVT_SVT", e1.r_dim, e1.r_type, e1.r_SVT, t,
+            e2.r_dim, e2.r_type, e2.r_SVT)
+    finally:
+        t.release()
+    like = e1 if any(d is not None for d in e1.dimnames) else e2
+    r = _ewise_result(ans, like)
+    r.warnings = warns
+    return r
+
+
+def _both_svt(e1, e2):
+    return isinstance(e1, SVT_SparseArray) and isinstance(e2, SVT_SparseArray)
+
+
 def Arith(e1, op, e2):
     """`e1 op e2` for op "*" or "/" where one side is an SVT_SparseArray and
     the other a numeric scalar or a vector of length nrow(x) (recycled along
@@ -380,7 +428,13 @@ def Arith(e1, op, e2):
     is `v / x` and every operation that would turn the implicit zeros into
     something else (`x * Inf`, `x * NA`, `x / 0`, "+", ...).  Served on the
     device: returns a new ResidentSVT (result type as in base R), with
-    `.warnings` holding R's warnings."""
+    `.warnings` holding R's warnings.
+
+    With two SVT_SparseArray operands of identical dimensions, op is "+",
+    "-" or "*": `as.matrix(e1) op as.matrix(e2)` with zeros dropped, integer
+    unless a side is double; "/", "^", "%%" and "%/%" are refused."""
+    if _both_svt(e1, e2):
+        return _ops2_call(e1, op, e2)
     if isinstance(e1, SVT_SparseArray):
         x, y, on_left = e1, e2, False
     elif isinstance(e2, SVT_SparseArray):
@@ -415,7 +469,13 @@ def Compare(e1, op, e2):
     implicit zeros stay FALSE (`x > 0`, `x >= 1`, `x == 3`, `x != 0`); any
     NA or NaN operand is refused.  Served on the device: returns a new
     ResidentSVT of type "logical" holding TRUE (and NA where x is NA or
-    NaN)."""
+    NaN).
+
+    With two SVT_SparseArray operands of identical dimensions, op is ">",
+    "<" or "!=" (`==`, `>=`, `<=` would make the implicit zeros TRUE and are
+    refused); NA or NaN on either side gives NA."""
+    if _both_svt(e1, e2):
+        return _ops2_call(e1, op, e2)
     if isinstance(e1, SVT_SparseArray):
         x, y, on_left = e1, e2, False
     elif isinstance(e2, SVT_SparseArray):
@@ -425,6 +485,17 @@ def Compare(e1, op, e2):
     n = np.asarray(y).size
     return _arith_call(x, op, y, 0 if n == 1 else 1, on_left,
                        "C_svtgpu_Compare_SVT")
+
+
+def Logic(e1, op, e2):
+    """`e1 & e2` / `e1 | e2` of two SVT_SparseArray objects of identical
+    dimensions: a new logical ResidentSVT, with base R's three-valued logic
+    (a nonzero value is TRUE, NA and NaN are NA).  A scalar or vector
+    operand is not supported."""
+    if not _both_svt(e1, e2):
+        raise TypeError("Logic on the GPU path needs two SVT_SparseArray "
+                        "operands")
+    return _ops2_call(e1, op, e2)
 
 
 def _is_call(x, fun):

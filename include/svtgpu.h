@@ -435,6 +435,32 @@ int svtgpu_ewise(svtgpu_matrix *x, int op, const void *operand,
 int svtgpu_ewise2(svtgpu_matrix *x, svtgpu_matrix *y, int op,
 		  svtgpu_matrix **out, int *warn);
 
+/* ---- subsetting ----
+ * x[i, j, ..., drop = FALSE] after R has normalised the subscripts: *out is a
+ * NEW matrix (owned by the caller) of n_rows x n_leaves with x's type, whose
+ * leaf k holds the entries of x's leaf leaves[k] at the rows rows[0 ..
+ * n_rows-1], renumbered to their positions in `rows` (offsets ascend in every
+ * leaf).  Host arrays of 0-based positions, any order, duplicates allowed;
+ * rows == NULL means every row (n_rows is then ignored), leaves == NULL every
+ * leaf (n_leaves ignored).  For an N-d array the caller passes as `leaves`
+ * the Cartesian product of the subscripts of dimensions 2..N in column-major
+ * order.  Values are copied bit for bit (NA, NaN payloads, stored +-0); a
+ * matrix without a value array gives a result without one.  The result
+ * carries no cached knowledge, and x (with its caches) is not modified.
+ * Routes, chosen from `rows`:
+ *   NULL or 0 .. nrow-1  one copy pass over the gathered leaves;
+ *   non-decreasing       a count pass over offsets and a row map, a scan,
+ *                        a write pass;
+ *   any other order      the non-decreasing route on sort(unique(rows)),
+ *                        then the device transpose, a leaf gather and the
+ *                        device transpose again, on matrices the size of the
+ *                        result; SVTGPU_ERR_UNSUPPORTED (naming the reason)
+ *                        where the transpose declines the intermediate.
+ * Ranges (and n_leaves < 2^31 - 1, else SVTGPU_ERR_UNSUPPORTED) are checked
+ * before a device is asked for; a failure leaves nothing allocated. */
+int svtgpu_subset(svtgpu_matrix *x, const int32_t *rows, int64_t n_rows,
+		  const int64_t *leaves, int64_t n_leaves, svtgpu_matrix **out);
+
 /* ---- synthetic data (benchmark inputs, generated in HBM) ----
  * Counter-based, so any leaf can be regenerated anywhere: with
  *   h  = mix64(seed + (cell + 1) * 0x9E3779B97F4A7C15),  cell = leaf*nrow + i

@@ -109,6 +109,7 @@ SIGNATURES = {
     "svtgpu_ewise": (_INT, [_P, _INT, _P, _INT, _I64, _INT, _INT,
                             _c.POINTER(_P), _c.POINTER(_INT)]),
     "svtgpu_ewise2": (_INT, [_P, _P, _INT, _c.POINTER(_P), _c.POINTER(_INT)]),
+    "svtgpu_subset": (_INT, [_P, _P, _I64, _P, _I64, _c.POINTER(_P)]),
 }
 
 # element-wise opcodes (SVTGPU_EW_*) and warning bits

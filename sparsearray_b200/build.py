@@ -25,10 +25,10 @@ LIBRSHIM = os.path.join(_SHIM, "librshim.so")
 CUDA_SOURCES = ["svtgpu_matrix.cu", "svtgpu_colstats.cu", "svtgpu_rowstats.cu",
                 "svtgpu_crossprod.cu", "svtgpu_transpose.cu",
                 "svtgpu_groupsum.cu", "svtgpu_gen.cu", "svtgpu_ewise.cu",
-                "svtgpu_medians.cu", "svtgpu_ewise2.cu"]
+                "svtgpu_medians.cu", "svtgpu_ewise2.cu", "svtgpu_subset.cu"]
 RGLUE_SOURCES = ["svt_flatten.c", "rglue_common.c", "rglue_matrixStats.c",
                  "rglue_mult.c", "rglue_summarization.c", "rglue_rowsum.c",
-                 "rglue_bridge.c", "rglue_ewise.c",
+                 "rglue_bridge.c", "rglue_ewise.c", "rglue_subset.c",
                  "rglue_init.c"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3",
               "-std=c++17", "-Xcompiler", "-fPIC,-fopenmp"]

@@ -157,6 +157,9 @@ int svtgpu_ensure_split(svtgpu_matrix *m, int nstrips, int strip_rows,
 			cudaStream_t s, const int32_t **split);
 int svtgpu_ensure_transpose(svtgpu_matrix *m, cudaStream_t s,
 			    svtgpu_matrix **out);
+/* the same, t(m) owned by the caller rather than cached in m */
+int svtgpu_transpose_fresh(svtgpu_matrix *m, cudaStream_t s,
+			   svtgpu_matrix **out);
 int svtgpu_launch_colstats(svtgpu_matrix *m, int opcode, int narm,
 			   double center, int64_t group, void *d_out,
 			   int32_t *d_warn, cudaStream_t stream);

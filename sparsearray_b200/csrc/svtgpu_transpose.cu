@@ -1501,3 +1501,14 @@ int svtgpu_ensure_transpose(svtgpu_matrix *m, cudaStream_t s,
 	*out = t;
 	return SVTGPU_OK;
 }
+
+/* t(m) for a matrix m that the caller built and is about to free: the
+ * transpose is handed to the caller (free it with svtgpu_matrix_free) instead
+ * of staying cached in m.  NULL + SVTGPU_OK as for svtgpu_ensure_transpose. */
+int svtgpu_transpose_fresh(svtgpu_matrix *m, cudaStream_t s,
+			   svtgpu_matrix **out)
+{
+	SVT_CHECK(svtgpu_ensure_transpose(m, s, out));
+	m->transposed = NULL;
+	return SVTGPU_OK;
+}

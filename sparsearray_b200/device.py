@@ -252,6 +252,33 @@ class DeviceSVT:
         out.warnings = [msg for bit, msg in N.EW_WARNINGS if warn.value & bit]
         return out
 
+    def subset(self, rows=None, leaves=None):
+        """`x[rows, leaves]` of this shard as a new owning DeviceSVT: 0-based
+        row positions and leaf positions local to the shard, any order,
+        duplicates allowed, None for all; see svtgpu_subset() in
+        include/svtgpu.h.  The result is a matrix of its own (leaf0 0)."""
+        L = N.lib()
+        r = l = None
+        if rows is not None:
+            r = np.ascontiguousarray(np.asarray(rows).reshape(-1),
+                                     dtype=np.int32)
+        if leaves is not None:
+            l = np.ascontiguousarray(np.asarray(leaves).reshape(-1),
+                                     dtype=np.int64)
+        h = ctypes.c_void_p()
+        N.check(L.svtgpu_subset(
+            self._h, None if r is None else r.ctypes.data_as(ctypes.c_void_p),
+            0 if r is None else r.size,
+            None if l is None else l.ctypes.data_as(ctypes.c_void_p),
+            0 if l is None else l.size, ctypes.byref(h)))
+        nnz = ctypes.c_int64(0)
+        N.check(L.svtgpu_matrix_info(h, None, None, ctypes.byref(nnz), None,
+                                     None))
+        return DeviceSVT(self.nrow if r is None else r.size,
+                         self.nleaf if l is None else l.size, nnz.value,
+                         self.val_type, None, None, None, handle=h,
+                         owns_handle=True)
+
     def download(self):
         """(leaf_ptr, offs, vals) of the shard on the host (vals None when
         the shard stores no values)."""

@@ -69,7 +69,8 @@ def registered_routines():
                  "C_svtgpu_set_cache",
                  "C_svtgpu_cache_stats", "C_svtgpu_Arith_SVT",
                  "C_svtgpu_Math_SVT", "C_svtgpu_Compare_SVT",
-                 "C_svtgpu_is_SVT", "C_svtgpu_Ops_SVT_SVT"):
+                 "C_svtgpu_is_SVT", "C_svtgpu_Ops_SVT_SVT",
+                 "C_svtgpu_subset_SVT"):
         n = ctypes.c_int(-1)
         p = L.rshim_lookup_call_routine(ctypes.byref(_info), name.encode(),
                                         ctypes.byref(n))

@@ -105,6 +105,7 @@ SEXP C_svtgpu_Compare_SVT(SEXP x_dim, SEXP x_type, SEXP x_SVT, SEXP op,
 SEXP C_svtgpu_is_SVT(SEXP x_dim, SEXP x_type, SEXP x_SVT, SEXP fun);
 SEXP C_svtgpu_Ops_SVT_SVT(SEXP x_dim, SEXP x_type, SEXP x_SVT, SEXP op,
 			  SEXP y_dim, SEXP y_type, SEXP y_SVT);
+SEXP C_svtgpu_subset_SVT(SEXP x_dim, SEXP x_type, SEXP x_SVT, SEXP Nindex);
 SEXP C_svtgpu_set_cache(SEXP on);
 SEXP C_svtgpu_cache_stats(void);
 SEXP C_get_num_procs(void);

@@ -73,6 +73,7 @@ static const R_CallMethodDef callMethods[] = {
 	CALLMETHOD_DEF(C_svtgpu_Compare_SVT, 7),
 	CALLMETHOD_DEF(C_svtgpu_is_SVT, 4),
 	CALLMETHOD_DEF(C_svtgpu_Ops_SVT_SVT, 7),
+	CALLMETHOD_DEF(C_svtgpu_subset_SVT, 4),
 	CALLMETHOD_DEF(C_svtgpu_set_cache, 1),
 	CALLMETHOD_DEF(C_svtgpu_cache_stats, 0),
 	{NULL, NULL, 0}

@@ -265,6 +265,22 @@ class SVT_SparseArray:
     def __le__(self, other):
         return Compare(self, "<=", other)
 
+    # -- subsetting; see subset() ---------------------------------------------
+    def __getitem__(self, key):
+        """`x[key]` with numpy's conventions, served by subset(): one key
+        per dimension (missing trailing ones mean all), each a 0-based int
+        (negative counts from the end), a slice, a 1-D integer array or a
+        boolean mask of exactly that extent.  Every dimension is kept, as
+        with R's `drop = FALSE`: `x[3]` has one row."""
+        if not isinstance(key, tuple):
+            key = (key,)
+        if len(key) > len(self.dim):
+            raise IndexError("too many indices: the array has %d dimensions"
+                             % len(self.dim))
+        key = key + (slice(None),) * (len(self.dim) - len(key))
+        return subset(self, [_numpy_key_to_subscript(k, n)
+                             for k, n in zip(key, self.dim)])
+
 
 class ResidentSVT(SVT_SparseArray):
     """An SVT_SparseArray whose SVT already lives in HBM: `r_SVT` is the
@@ -566,6 +582,93 @@ def to_csc(x, as_ngCMatrix=False):
                    else np.array(rshim.to_numpy(elts[k])[0]))
     rshim.lib().rshim_release_tree(ans)
     return tuple(out)
+
+
+def _numpy_key_to_subscript(k, n):
+    """one numpy-style key along an extent n -> a 1-based int32 vector, or
+    None for all of the dimension in order"""
+    if isinstance(k, slice):
+        idx = np.arange(*k.indices(n), dtype=np.int64)
+        if idx.size == n and (n == 0 or (idx[0] == 0 and k.step in (None, 1))):
+            return None
+    elif isinstance(k, (bool, np.bool_)):
+        raise IndexError("a boolean scalar is not a subscript")
+    elif isinstance(k, (int, np.integer)):
+        idx = np.array([int(k)], np.int64)
+    else:
+        a = np.asarray(k)
+        if a.ndim != 1:
+            raise IndexError("only 1-D index arrays are supported")
+        if a.dtype.kind == "b":
+            if a.size != n:
+                raise IndexError("boolean index of length %d does not match "
+                                 "the extent %d" % (a.size, n))
+            idx = np.flatnonzero(a)
+        elif a.dtype.kind in "iu" or a.size == 0:
+            idx = a.astype(np.int64)
+        else:
+            raise IndexError("index arrays must hold integers or booleans")
+    if idx.size and (idx.min() < -n or idx.max() >= n):
+        raise IndexError("index out of bounds for an extent of %d" % n)
+    return (np.where(idx < 0, idx + n, idx) + 1).astype(np.int32)
+
+
+def subset(x, Nindex):
+    """`x[i, j, ..., drop = FALSE]` after R's normalisation of the
+    subscripts: Nindex has one element per dimension, None (all of it, in
+    order) or a vector of 1-based integer positions in any order, with
+    duplicates repeating the row / column and a zero-length vector giving an
+    extent of 0.  Served on the device by C_svtgpu_subset_SVT: returns a new
+    ResidentSVT of x's type, with dimension lengths(Nindex) and dimnames
+    subset the same way; values are copied bit for bit.  NA in a subscript
+    ("subscript contains NAs") and positions outside [1, dim(x)[k]]
+    ("subscript contains out-of-bounds indices") are refused, as are
+    non-integer subscripts and an Nindex of the wrong length."""
+    if not isinstance(x, SVT_SparseArray):
+        raise TypeError("'x' must be an SVT_SparseArray")
+    temps = []
+    try:
+        if isinstance(Nindex, (list, tuple)):
+            elts = []
+            for s in Nindex:
+                if s is None:
+                    elts.append(None)
+                    continue
+                a = np.asarray(s).reshape(-1)
+                if a.dtype.kind in "iu" or a.size == 0:
+                    r = rshim.wrap(a.astype(np.int32), rshim.INTSXP)
+                elif a.dtype.kind == "b":
+                    r = rshim.wrap(a.astype(np.int32), rshim.LGLSXP)
+                else:
+                    r = rshim.wrap(a.astype(np.float64), rshim.REALSXP)
+                elts.append(r)
+            nidx = rshim.rlist(elts)
+        elif isinstance(Nindex, str):
+            nidx = rshim.string(Nindex)
+        else:
+            nidx = _operand(Nindex)
+        temps.append(nidx)
+        ans, warns = rcall.SparseArray_Call("C_svtgpu_subset_SVT", x.r_dim,
+                                            x.r_type, x.r_SVT, nidx)
+    finally:
+        for t in temps:
+            t.release()
+    dim, dimnames = [], []
+    for k, s in enumerate(Nindex):
+        names = x.dimnames[k]
+        if s is None:
+            dim.append(x.dim[k])
+            dimnames.append(names)
+        else:
+            s = np.asarray(s).reshape(-1)
+            dim.append(s.size)
+            dimnames.append(None if names is None
+                            else [names[i - 1] for i in s])
+    like = SVT_SparseArray.__new__(SVT_SparseArray)
+    like.dim, like.dimnames = tuple(dim), dimnames
+    r = _ewise_result(ans, like)
+    r.warnings = warns
+    return r
 
 
 SVT_SparseMatrix = SVT_SparseArray

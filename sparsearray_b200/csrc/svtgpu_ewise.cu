@@ -13,7 +13,7 @@
  * cyclically (block b: tiles b, b + G, ...), so the GPU sweeps the arrays
  * front to back as row_hist does, with 16-byte loads and stores of four
  * entries per lane.  Per-column operands find the leaf of each tile's first
- * and last entry by binary search, as hist_tile_leaves does, then the leaf of
+ * and last entry by binary search, as tile_leaves does, then the leaf of
  * each group of four inside those bounds.  Warnings and "a value became 0"
  * are OR-ed into one device word.
  *

@@ -45,11 +45,12 @@ struct svtgpu_matrix {
 	int split_tile_rows[SVTGPU_NSPLIT];
 	int split_ntiles[SVTGPU_NSPLIT];
 	int split_next;
-	/* row_hist, cyclic form: the leaf that holds the first entry of every
-	   tile of hist_tile entries, and the most leaves a tile touches */
-	int64_t *d_hist_tiles;
-	int64_t hist_tile, hist_ntiles;
-	int hist_max_leaves;
+	/* tile table (svt_ensure_tile_table): the leaf that holds the first
+	   entry of every tile of tile_entries entries, and the most leaves a
+	   tile touches */
+	int64_t *d_tile_leaf;
+	int64_t tile_entries, tile_count;
+	int tile_max_leaves;
 	int64_t vmax_abs;    /* max |x| of an integer matrix, -1 = not computed */
 	/* value payloads committed as int8 / at native width: a matrix that
 	   only ever saw int8 payloads has |x| <= 127 without looking */
@@ -98,6 +99,17 @@ struct svtgpu_matrix {
 int svt_ensure_compact(svtgpu_matrix *m, cudaStream_t s);
 /* Free the compact copy (stream-ordered on s) and forget that it was decided. */
 void svt_drop_compact(svtgpu_matrix *m, cudaStream_t s);
+
+/* ---- tile table ----
+ * The cyclic form of row_hist cuts the entries into tiles of `tile` entries
+ * and lets the CTAs take them round-robin, so that the whole GPU sweeps the
+ * arrays front to back.  m->d_tile_leaf[t] (t <= ntiles) is the leaf that
+ * holds entry min(t * tile, nnz - 1): tile t touches leaves d_tile_leaf[t] ..
+ * d_tile_leaf[t + 1], and m->tile_max_leaves is the most leaves any tile
+ * touches.  Built once per matrix and tile size (synchronises s once).
+ * SVT_TILE_ENTRIES is the tile of the value modes.  Requires nnz > 0. */
+#define SVT_TILE_ENTRIES 32768
+int svt_ensure_tile_table(svtgpu_matrix *m, int64_t tile, cudaStream_t s);
 
 /* upper bound of |x| over the non-NA values of an integer matrix when one is
    known without a pass over the data, else -1 */

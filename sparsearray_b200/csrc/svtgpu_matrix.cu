@@ -537,7 +537,7 @@ extern "C" int svtgpu_matrix_free(svtgpu_matrix *m)
 	if (m->d_scratch) svt_free_async(m->d_scratch, 0);
 	for (int i = 0; i < SVTGPU_NSPLIT; i++)
 		if (m->d_split[i]) svt_free_async(m->d_split[i], 0);
-	if (m->d_hist_tiles) svt_free_async(m->d_hist_tiles, 0);
+	if (m->d_tile_leaf) svt_free_async(m->d_tile_leaf, 0);
 	svt_drop_compact(m, 0);
 	cudaDeviceSynchronize();
 	if (m->up_begin) cudaEventDestroy(m->up_begin);
@@ -644,10 +644,10 @@ extern "C" int svtgpu_matrix_fold_rows(svtgpu_matrix *m, int64_t fold)
 			svt_free_async(m->d_split[i], s);
 		m->d_split[i] = NULL;
 	}
-	if (m->d_hist_tiles != NULL)
-		svt_free_async(m->d_hist_tiles, s);
-	m->d_hist_tiles = NULL;
-	m->hist_tile = 0;
+	if (m->d_tile_leaf != NULL)
+		svt_free_async(m->d_tile_leaf, s);
+	m->d_tile_leaf = NULL;
+	m->tile_entries = 0;
 	/* the compact offsets hold the old rows (and nrow may now exceed
 	   what 16 bits can hold) */
 	svt_drop_compact(m, s);
@@ -1075,6 +1075,62 @@ int svt_ensure_compact(svtgpu_matrix *m, cudaStream_t s)
 	/* later calls may come on other streams */
 	SVT_CUDA(cudaStreamSynchronize(s));
 	m->compact_state = SVT_COMPACT_BUILT;
+	return SVTGPU_OK;
+}
+
+/* ---- tile table (svtgpu_internal.h) ---- */
+__global__ void __launch_bounds__(256)
+tile_leaves(const int64_t *__restrict__ leaf_ptr, int64_t nleaf, int64_t nnz,
+	    int64_t tile, int64_t ntiles, int64_t *__restrict__ tile_leaf,
+	    int *max_leaves, int pass)
+{
+	const int64_t t = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
+	if (t > ntiles)
+		return;
+	if (pass == 0) {
+		int64_t e = t * tile;
+		if (e > nnz - 1) e = nnz - 1;
+		/* first leaf whose range ends after entry e */
+		int64_t lo = 0, hi = nleaf;
+		while (lo < hi) {
+			const int64_t mid = lo + ((hi - lo) >> 1);
+			if (leaf_ptr[mid + 1] <= e) lo = mid + 1;
+			else                        hi = mid;
+		}
+		tile_leaf[t] = lo;
+	} else if (t < ntiles) {
+		const int64_t L = tile_leaf[t + 1] - tile_leaf[t] + 1;
+		atomicMax(max_leaves, L > INT32_MAX ? INT32_MAX : (int) L);
+	}
+}
+
+int svt_ensure_tile_table(svtgpu_matrix *m, int64_t tile, cudaStream_t s)
+{
+	if (m->d_tile_leaf != NULL && m->tile_entries == tile)
+		return SVTGPU_OK;
+	if (m->d_tile_leaf != NULL)
+		svt_free_async(m->d_tile_leaf, s);
+	m->d_tile_leaf = NULL;
+	m->tile_entries = 0;
+	const int64_t ntiles = (m->nnz + tile - 1) / tile;
+	SVT_CUDA(svt_malloc_async((void **) &m->d_tile_leaf,
+				  8 * (size_t) (ntiles + 1) + 64, s));
+	int *d_max = (int *) (m->d_tile_leaf + ntiles + 1);
+	SVT_CUDA(cudaMemsetAsync(d_max, 0, sizeof(int), s));
+	const unsigned g = (unsigned) ((ntiles + 1 + 255) / 256);
+	tile_leaves<<<g, 256, 0, s>>>(m->d_leaf_ptr, m->nleaf, m->nnz, tile,
+				      ntiles, m->d_tile_leaf, d_max, 0);
+	tile_leaves<<<g, 256, 0, s>>>(m->d_leaf_ptr, m->nleaf, m->nnz, tile,
+				      ntiles, m->d_tile_leaf, d_max, 1);
+	SVT_CUDA(cudaGetLastError());
+	svtgpu_count_launch(2);
+	int h_max = 0;
+	SVT_CUDA(cudaMemcpyAsync(&h_max, d_max, sizeof(int),
+				 cudaMemcpyDeviceToHost, s));
+	SVT_CUDA(cudaStreamSynchronize(s));
+	m->tile_entries = tile;
+	m->tile_count = ntiles;
+	m->tile_max_leaves = h_max;
 	return SVTGPU_OK;
 }
 

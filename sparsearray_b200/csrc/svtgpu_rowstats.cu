@@ -1711,55 +1711,60 @@ row_hist(RowHistParams P)
 			hist_red(cell_s + (o << 2), (unsigned int) x);
 		}
 	};
+	/* 8 entries: one 16-byte load of offsets and one 8-byte load of values */
+	auto add8_group = [&](const int4 o, const uint2 v) {
+		const uint32_t ow[4] = { (uint32_t) o.x, (uint32_t) o.y,
+					 (uint32_t) o.z, (uint32_t) o.w };
+		const uint32_t vw[2] = { v.x, v.y };
+#pragma unroll
+		for (int j = 0; j < 8; j++)
+			add8((ow[j >> 1] >> ((j & 1) * 16)) & 0xFFFFu,
+			     (int) (int8_t) (vw[j >> 2] >> ((j & 3) * 8)));
+	};
+	/* entries per batch of the compact stream: every thread takes K8
+	   groups of 8 */
+	constexpr int K8 = 2;
+	constexpr int64_t BATCH8 = (int64_t) HIST_THREADS * 8 * K8;
 	auto stream8 = [&](const int64_t start, const int64_t end) {
-	/* single entries up to a multiple of 8, then batches in which every
-	   thread takes K groups of 8 entries (one 16-byte load of offsets and
-	   one 8-byte load of values each), double-buffered as above */
-	constexpr int K = 2;
+	/* single entries up to a multiple of 8, then full batches,
+	   double-buffered as above */
 	int64_t head = (8 - (start & 7)) & 7;
 	if (head > end - start)
 		head = end - start;
 	if ((int64_t) threadIdx.x < head)
 		add8(P.offs16[start + threadIdx.x], P.vals8[start + threadIdx.x]);
 	const int64_t vstart = start + head;
-	const int64_t nfull = (end - vstart) / ((int64_t) HIST_THREADS * 8 * K);
+	const int64_t nfull = (end - vstart) / BATCH8;
 	const int4 *po = (const int4 *) (P.offs16 + vstart) + threadIdx.x;
 	const uint2 *pv = (const uint2 *) (P.vals8 + vstart) + threadIdx.x;
-	int4 o_nx[K];
-	uint2 v_nx[K];
+	int4 o_nx[K8];
+	uint2 v_nx[K8];
 	auto request = [&]() {
 #pragma unroll
-		for (int k = 0; k < K; k++) {
+		for (int k = 0; k < K8; k++) {
 			o_nx[k] = ldg_stream_v4(po + k * HIST_THREADS);
 			v_nx[k] = ldg_stream_v2(pv + k * HIST_THREADS);
 		}
-		po += K * HIST_THREADS;
-		pv += K * HIST_THREADS;
+		po += K8 * HIST_THREADS;
+		pv += K8 * HIST_THREADS;
 	};
 	if (nfull > 0)
 		request();
 	for (int64_t b = 0; b < nfull; b++) {
-		int4 o[K];
-		uint2 v[K];
+		int4 o[K8];
+		uint2 v[K8];
 #pragma unroll
-		for (int k = 0; k < K; k++) {
+		for (int k = 0; k < K8; k++) {
 			o[k] = o_nx[k];
 			v[k] = v_nx[k];
 		}
 		if (b + 1 < nfull)
 			request();
 #pragma unroll
-		for (int k = 0; k < K; k++) {
-			const uint32_t ow[4] = { (uint32_t) o[k].x, (uint32_t) o[k].y,
-						 (uint32_t) o[k].z, (uint32_t) o[k].w };
-			const uint32_t vw[2] = { v[k].x, v[k].y };
-#pragma unroll
-			for (int j = 0; j < 8; j++)
-				add8((ow[j >> 1] >> ((j & 1) * 16)) & 0xFFFFu,
-				     (int) (int8_t) (vw[j >> 2] >> ((j & 3) * 8)));
-		}
+		for (int k = 0; k < K8; k++)
+			add8_group(o[k], v[k]);
 	}
-	for (int64_t e = vstart + nfull * HIST_THREADS * 8 * K + threadIdx.x;
+	for (int64_t e = vstart + nfull * BATCH8 + threadIdx.x;
 	     e < end; e += HIST_THREADS)
 		add8(P.offs16[e], P.vals8[e]);
 	};
@@ -1852,6 +1857,32 @@ row_hist(RowHistParams P)
 			la = P.tile_leaf[t];
 			lb = P.tile_leaf[t + 1];
 		}
+		/* NARROW: the CTA's tiles are one continuous stream -- the first
+		   batch of its next tile is requested before the last batch of
+		   this one is added, so no tile starts with an empty pipeline
+		   (the loads write registers, not cells, so the look at the
+		   cells between tiles can sit in between).  Groups of 8 past
+		   the last entry read as zeros and add nothing; the one that
+		   holds it reads the copy's zeroed padding. */
+		constexpr int NB8 = (int) (SVT_TILE_ENTRIES / BATCH8);
+		static_assert(SVT_TILE_ENTRIES % BATCH8 == 0, "tile of batches");
+		int4 o_nx[K8];
+		uint2 v_nx[K8];
+		auto request8 = [&](const int64_t e) {
+			const int4 *po = (const int4 *) (P.offs16 + e) + threadIdx.x;
+			const uint2 *pv = (const uint2 *) (P.vals8 + e) + threadIdx.x;
+#pragma unroll
+			for (int k = 0; k < K8; k++) {
+				const bool ok = e + ((int64_t) k * HIST_THREADS +
+						     threadIdx.x) * 8 < P.nnz;
+				o_nx[k] = ok ? ldg_stream_v4(po + k * HIST_THREADS)
+					     : make_int4(0, 0, 0, 0);
+				v_nx[k] = ok ? ldg_stream_v2(pv + k * HIST_THREADS)
+					     : make_uint2(0, 0);
+			}
+		};
+		if (NARROW && t < P.ntiles)
+			request8(t * P.tile);
 		while (t < P.ntiles) {
 			const int64_t L = lb - la + 1;
 			const int64_t tn = t + gridDim.x;
@@ -1866,8 +1897,28 @@ row_hist(RowHistParams P)
 			}
 			used += L;
 			const int64_t start = t * P.tile;
-			feed(start, start + P.tile < P.nnz ? start + P.tile
-							   : P.nnz);
+			if (NARROW) {
+#pragma unroll
+				for (int b = 0; b < NB8; b++) {
+					int4 o[K8];
+					uint2 v[K8];
+#pragma unroll
+					for (int k = 0; k < K8; k++) {
+						o[k] = o_nx[k];
+						v[k] = v_nx[k];
+					}
+					if (b + 1 < NB8)
+						request8(start + (b + 1) * BATCH8);
+					else if (tn < P.ntiles)
+						request8(tn * P.tile);
+#pragma unroll
+					for (int k = 0; k < K8; k++)
+						add8_group(o[k], v[k]);
+				}
+			} else {
+				feed(start, start + P.tile < P.nnz ? start + P.tile
+								   : P.nnz);
+			}
 			t = tn;
 			la = na;
 			lb = nb;
@@ -1908,33 +1959,6 @@ row_hist(RowHistParams P)
 			feed(P.leaf_ptr[p0], P.leaf_ptr[p1]);
 			checkpoint(p1 == bounds[1]);
 		}
-	}
-}
-
-/* tile_leaf[t] = the leaf that holds entry t * tile (t = ntiles: the last
-   leaf); *max_leaves = the most leaves any tile touches */
-__global__ void __launch_bounds__(256)
-hist_tile_leaves(const int64_t *__restrict__ leaf_ptr, int64_t nleaf,
-		 int64_t nnz, int64_t tile, int64_t ntiles,
-		 int64_t *__restrict__ tile_leaf, int *max_leaves, int pass)
-{
-	const int64_t t = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
-	if (t > ntiles)
-		return;
-	if (pass == 0) {
-		int64_t e = t * tile;
-		if (e > nnz - 1) e = nnz - 1;
-		/* first leaf whose range ends after entry e */
-		int64_t lo = 0, hi = nleaf;
-		while (lo < hi) {
-			const int64_t mid = lo + ((hi - lo) >> 1);
-			if (leaf_ptr[mid + 1] <= e) lo = mid + 1;
-			else                        hi = mid;
-		}
-		tile_leaf[t] = lo;
-	} else if (t < ntiles) {
-		const int64_t L = tile_leaf[t + 1] - tile_leaf[t] + 1;
-		atomicMax(max_leaves, L > INT32_MAX ? INT32_MAX : (int) L);
 	}
 }
 
@@ -1983,36 +2007,14 @@ int launch_row_hist(svtgpu_matrix *m, int mode, int64_t max_abs,
 	/* the cyclic form (tiles of 4 batches, round-robin over the SMs) when
 	   there are at least 4 tiles per SM and no tile touches more leaves
 	   than a cell can take; the tile table is built once per matrix */
-	const int64_t tile = (int64_t) HIST_THREADS * (lac ? 16 : 8) * 4;
+	const int64_t tile = lac ? (int64_t) HIST_THREADS * 16 * 4
+				 : (int64_t) SVT_TILE_ENTRIES;
 	const int64_t ntiles = (m->nnz + tile - 1) / tile;
 	if (ntiles >= (int64_t) sms * 4 &&
 	    strcmp(svtgpu_env("SVTGPU_ROW_HIST_TILES", "cyclic"), "cyclic") == 0) {
-		if (m->d_hist_tiles == NULL || m->hist_tile != tile) {
-			if (m->d_hist_tiles != NULL)
-				svt_free_async(m->d_hist_tiles, s);
-			m->d_hist_tiles = NULL;
-			int *d_max = NULL;
-			SVT_CUDA(svt_malloc_async((void **) &m->d_hist_tiles,
-					8 * (size_t) (ntiles + 1) + 64, s));
-			d_max = (int *) (m->d_hist_tiles + ntiles + 1);
-			SVT_CUDA(cudaMemsetAsync(d_max, 0, sizeof(int), s));
-			const unsigned g = (unsigned) ((ntiles + 1 + 255) / 256);
-			hist_tile_leaves<<<g, 256, 0, s>>>(m->d_leaf_ptr, m->nleaf,
-				m->nnz, tile, ntiles, m->d_hist_tiles, d_max, 0);
-			hist_tile_leaves<<<g, 256, 0, s>>>(m->d_leaf_ptr, m->nleaf,
-				m->nnz, tile, ntiles, m->d_hist_tiles, d_max, 1);
-			SVT_CUDA(cudaGetLastError());
-			svtgpu_count_launch(2);
-			int h_max = 0;
-			SVT_CUDA(cudaMemcpyAsync(&h_max, d_max, sizeof(int),
-					cudaMemcpyDeviceToHost, s));
-			SVT_CUDA(cudaStreamSynchronize(s));
-			m->hist_tile = tile;
-			m->hist_ntiles = ntiles;
-			m->hist_max_leaves = h_max;
-		}
-		if (m->hist_max_leaves <= P.piece_leaves) {
-			P.tile_leaf = m->d_hist_tiles;
+		SVT_CHECK(svt_ensure_tile_table(m, tile, s));
+		if (m->tile_max_leaves <= P.piece_leaves) {
+			P.tile_leaf = m->d_tile_leaf;
 			P.tile = tile;
 			P.ntiles = ntiles;
 			grid = sms;

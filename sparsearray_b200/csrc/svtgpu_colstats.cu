@@ -528,11 +528,13 @@ colstats_direct(ColParams P)
 
 /* ------------------------------------------------------------------------
  * colstats_sum_i8: the integer SUM class (colSums, colMeans) over the compact
- * int8 values (svtgpu_internal.h).  A warp per segment, 16-byte loads over
- * the aligned middle with up to four per lane in flight, single bytes at the
- * ends.  Per 32-bit word __dp4a gives the signed byte sum, in which every NA
- * byte (-128) counts -128, and __vcmpeq4 marks the NA bytes (0xFF each), so
- * sum = dp4a + 128 #NA exactly: the partial equals the wide kernel's.
+ * int8 values (svtgpu_internal.h).  A warp per segment reads the 16-byte
+ * words that cover it, the partial words at either end included, with up to
+ * SUM_I8_UNROLL loads per lane in flight: a C2 leaf (~2.3 KB) costs one round
+ * trip.  The bytes of the end words outside the segment are masked.  Per
+ * 32-bit word __dp4a(w, 0x01010101) gives the signed byte sum, in which every
+ * NA byte (-128) counts -128, and __vcmpeq4 marks the NA bytes (0xFF each),
+ * so sum = dp4a + 128 #NA exactly: the partial equals the wide kernel's.
  */
 __device__ __forceinline__ void sum_i8_word(uint32_t w, int &s, int &na_bits)
 {
@@ -540,14 +542,30 @@ __device__ __forceinline__ void sum_i8_word(uint32_t w, int &s, int &na_bits)
 	na_bits += __popc(__vcmpeq4(w, 0x80808080u));
 }
 
-#define SUM_I8_BLOCKS_PER_SM 6   /* 40 registers: four 16-byte loads in flight */
+/* bytes [a, b) (0 <= a <= b <= 16) of a 16-byte word */
+__device__ __forceinline__ void sum_i8_masked(uint4 u, int a, int b, int &s,
+					      int &na_bits)
+{
+	const uint32_t w[4] = {u.x, u.y, u.z, u.w};
+#pragma unroll
+	for (int j = 0; j < 4; j++) {
+		const int lo = min(max(a - 4 * j, 0), 4);
+		const int hi = min(max(b - 4 * j, 0), 4);
+		const uint32_t mhi = hi == 4 ? 0xFFFFFFFFu : (1u << (8 * hi)) - 1;
+		const uint32_t mlo = lo == 4 ? 0xFFFFFFFFu : (1u << (8 * lo)) - 1;
+		sum_i8_word(w[j] & mhi & ~mlo, s, na_bits);
+	}
+}
+
+#define SUM_I8_BLOCKS_PER_SM 4   /* 64 registers, no spills */
+#define SUM_I8_UNROLL 5      /* 2.5 KB per warp and round trip */
 __global__ void __launch_bounds__(256, SUM_I8_BLOCKS_PER_SM)
 colstats_sum_i8(ColParams P, const int8_t *__restrict__ v8)
 {
 	const int lane = threadIdx.x & 31;
 	const int64_t warps = ((int64_t) gridDim.x * blockDim.x) >> 5;
 	const int64_t gw = ((int64_t) blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-	/* a C2 leaf is ~2.3 KB: its bounds are requested a segment ahead */
+	/* the bounds are requested a segment ahead */
 	int64_t nstart = 0, nend = 0;
 	if (gw < P.nseg) {
 		nstart = P.leaf_ptr[gw * P.group];
@@ -559,42 +577,38 @@ colstats_sum_i8(ColParams P, const int8_t *__restrict__ v8)
 			nstart = P.leaf_ptr[(seg + warps) * P.group];
 			nend = P.leaf_ptr[(seg + warps + 1) * P.group];
 		}
+		/* words w0 .. w0 + nw - 1 cover the segment; its bytes are
+		   [a, 16) of the first and [0, b) of the last.  Rounding out
+		   to 16 bytes stays inside the copy (SVT_COMPACT_PAD). */
+		const int64_t w0 = start >> 4;
+		const int nw = (int) (((end + 15) >> 4) - w0);
+		const int a = (int) (start & 15);
+		const int b = (int) (end - ((w0 + nw - 1) << 4));
+		const uint4 *q = (const uint4 *) v8 + w0;
 		long long sum = 0;
 		int na_bits = 0;   /* 8 per NA */
-		const int64_t a16 = (start + 15) & ~(int64_t) 15;
-		const int64_t b16 = end & ~(int64_t) 15;
-		int64_t lo = start, hi = end;   /* bytes left to single lanes */
-		if (a16 < b16) {
-			const uint4 *q = (const uint4 *) (v8 + a16);
-			const int nv = (int) ((b16 - a16) >> 4);
-			for (int i = lane; i < nv; i += 128) {
-				uint4 u[4];
+		for (int i = lane; i < nw; i += 32 * SUM_I8_UNROLL) {
+			uint4 u[SUM_I8_UNROLL];
 #pragma unroll
-				for (int k = 0; k < 4; k++)
-					u[k] = i + 32 * k < nv ? __ldcs(q + i + 32 * k)
-							       : make_uint4(0, 0, 0, 0);
-				int s = 0;
+			for (int k = 0; k < SUM_I8_UNROLL; k++)
+				u[k] = i + 32 * k < nw ? __ldcs(q + i + 32 * k)
+						       : make_uint4(0, 0, 0, 0);
+			int s = 0;
 #pragma unroll
-				for (int k = 0; k < 4; k++) {
+			for (int k = 0; k < SUM_I8_UNROLL; k++) {
+				const int wi = i + 32 * k;
+				if (wi == 0 || wi == nw - 1) {
+					sum_i8_masked(u[k], wi == 0 ? a : 0,
+						      wi == nw - 1 ? b : 16, s,
+						      na_bits);
+				} else {
 					sum_i8_word(u[k].x, s, na_bits);
 					sum_i8_word(u[k].y, s, na_bits);
 					sum_i8_word(u[k].z, s, na_bits);
 					sum_i8_word(u[k].w, s, na_bits);
 				}
-				sum += s;
 			}
-			/* < 16 bytes at either end */
-			if (start + lane < a16) {
-				const int x = v8[start + lane];
-				sum += x;
-				na_bits += x == SVT_COMPACT_NA_I8 ? 8 : 0;
-			}
-			lo = b16;
-		}
-		for (int64_t e = lo + lane; e < hi; e += 32) {
-			const int x = v8[e];
-			sum += x;
-			na_bits += x == SVT_COMPACT_NA_I8 ? 8 : 0;
+			sum += s;
 		}
 		const long long n_na = svt_warp_sum((long long) na_bits) >> 3;
 		sum = svt_warp_sum(sum) + 128 * n_na;
